@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            (N > 1: launched by torch.distributed.run, one rank / GPU)
     python bench.py --impl reference ...                     (the reference's CPU path: cv2 LK + the BA oracle port)
+    python bench.py ... --dump-outputs DIR                   (+ what the headline path returned in its last timed step, DIR/<name>.npy)
 
 A "step" = one frame of every one of B independent 1280x560 synthetic streams resident on this GPU:
 pyramid build (levels 1..3) of the B new frames + fused forward/backward KLT of 300 points per stream
@@ -54,6 +55,8 @@ def parse():
     ap.add_argument("--no-clahe", action="store_true", help="skip the CLAHE section")
     ap.add_argument("--no-keyframe", action="store_true", help="skip the full-keyframe-path line")
     ap.add_argument("--no-e2e-pipeline", action="store_true", help="e2e: one set of solver handles (the host packs and the GPU solves in turn)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the arrays the headline path returned in its last timed step to DIR/<name>.npy "
+                                                          "(rank 0; float32 / float64; a fixed sample of the streams beyond 64 MB)")
     return ap.parse_args()
 
 
@@ -77,6 +80,20 @@ def pair_points(pts, fa, fb, seed):
     prev = pts[fa].astype(np.float32)
     init = (pts[fb] + rng.normal(0.0, 1.0, size=pts[fb].shape)).astype(np.float32)
     return prev, init
+
+
+def write_outputs(out_dir, arrays, limit=64 << 20):
+    """Save each array (leading axis = stream) as out_dir/<name>.npy, float64 kept and everything else as float32.  Beyond `limit` bytes in
+    all, every array keeps the same seeded sample of streams, so that two builds run with the same arguments stay comparable."""
+    arrays = {k: a.astype(np.float64 if a.dtype == np.float64 else np.float32) for k, a in arrays.items()}
+    n = len(next(iter(arrays.values())))
+    per_stream = sum(a.nbytes for a in arrays.values()) / n
+    if per_stream * n > limit:
+        keep = np.sort(np.random.default_rng(0).choice(n, int(limit // per_stream), replace=False))
+        arrays = {k: a[keep] for k, a in arrays.items()}
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
 
 
 # ----------------------------------------------------------------------------------------------- clocks sampler
@@ -127,7 +144,7 @@ def cpu_arm_inputs(frames, pts, n_probs=4):
     for k in range(10):
         prev, init = pair_points(pts, seq[k], seq[k + 1], 99 + k)
         pairs.append((seq[k], seq[k + 1], prev, init))
-    olib = C.CDLL(oracle.build())
+    olib = C.CDLL(oracle.LIB)  # built by __graft_entry__.build(): the bench only reads the source tree
     oa.declare(olib)
     oa.declare_ba(olib)
     probs = make_windows(n_probs, lambda *a: oa.preintegrate(olib, *a))
@@ -167,7 +184,7 @@ def cpu_single_stream(frames, pts, seconds: float = 1.5):
         klt = k / (time.perf_counter() - t0)
     except Exception:
         pass
-    olib = C.CDLL(oracle.build())
+    olib = C.CDLL(oracle.LIB)
     oa.declare(olib)
     oa.declare_ba(olib)
     prob = make_windows(1, lambda *a: oa.preintegrate(olib, *a))[0]
@@ -449,6 +466,28 @@ def run_b200(args):
             dist.barrier()
         torch.cuda.synchronize()
 
+    def headline_outputs():
+        """What the last step_resident handed its caller, one row per stream: the fused LK results and, per window, the solved parameters
+        with the pass-2 summary.  The solvers download into copies: the uploaded windows feed the later sections unchanged."""
+        out = {"klt_fwd_xy": d_fwd.cpu().numpy().reshape(B, NPTS, 2), "klt_bwd_xy": d_bwd.cpu().numpy().reshape(B, NPTS, 2),
+               "klt_status": d_st.cpu().numpy().reshape(B, NPTS)}
+        if use_ba:
+            par = ("pose", "mix", "ext", "invdepth")
+            got = {q: [] for q in par + ("final_cost", "iterations")}
+            for k, sv in enumerate(solvers):
+                part = [dict(w_, **{q: np.array(w_[q], np.float64) for q in par}) for w_ in windows[bounds[k]:bounds[k + 1]]]
+                arr, summ = (BaProblem * len(part))(*[to_struct(w_) for w_ in part]), (BaSummary * len(part))()
+                if lib().icg_ba_download(sv._h, len(part), arr, summ) != 0:
+                    raise RuntimeError(lib().icg_last_error().decode())
+                for w_, s_ in zip(part, summ):
+                    for q in par:
+                        got[q].append(w_[q])
+                    got["final_cost"].append(s_.final_cost)
+                    got["iterations"].append(s_.iterations)
+            out.update({"ba_" + q: np.array(v, np.float64) for q, v in got.items()})
+            out["ba_pose"], out["ba_mix"] = out["ba_pose"].reshape(B, -1, 7), out["ba_mix"].reshape(B, -1, 9)
+        return out
+
     def timed(step_fn, mode="step", finish_fn=None):
         for s in range(args.warmup):
             if step_fn is not None:
@@ -506,6 +545,8 @@ def run_b200(args):
     with ClockSampler(local_rank) as clk:
         ms_res, _ = timed(step_resident)
         launches = int(lib().icg_launch_count())
+        if args.dump_outputs and rank == 0:
+            write_outputs(args.dump_outputs, headline_outputs())
         ms_e2e, _ = timed(step_e2e, finish_fn=e2e_finish)
         _, kms = timed(klt_resident, mode="klt_kernel")
         bms = timed(None, mode="ba_only")[1] if use_ba else []
@@ -640,7 +681,7 @@ def run_b200(args):
             import ctypes as C
             import oracle
             from tests import oracle_api as oa
-            olib = C.CDLL(oracle.build())
+            olib = C.CDLL(oracle.LIB)
             oa.declare_ba(olib)
             pw = make_windows(1, lambda *a: oa.preintegrate(olib, *a))[0]
             oa.ba_marginalize(olib, pw, 1)

@@ -4,8 +4,8 @@
 What runs: per frame of one stream, the reference's front-end calls on cv2 (the OpenCV the reference links: forward + backward
 `calcOpticalFlowPyrLK` as IG/tracking/tracking.cc:385-403 calls it) and one `gvinsOptimization` window solve (5 LM iterations, chi-square
 culling, 15 iterations; IG/ic_gvins.cc:1130-1239) on the BA PORT (oracle/ba_ref.cpp -- Ceres is neither vendored nor installed, so this
-leg is our restatement, compiled `-O3 -march=native` into oracle/_perf/ on the machine that runs it; the parity copy keeps
-`-O2 -ffp-contract=off`).
+leg is our restatement, compiled `-O3 -march=native` into a temporary directory on the machine that runs it, so that the source
+tree is only read; the parity copy keeps `-O2 -ffp-contract=off`).
 
 How it is measured (throughput mode, like the GPU arm: independent streams):
   * one PROCESS per usable core (spawn), each pinned with os.sched_setaffinity to its own core, cv2 / the port single-threaded inside;
@@ -16,7 +16,6 @@ How it is measured (throughput mode, like the GPU arm: independent streams):
 from __future__ import annotations
 
 import ctypes as C
-import hashlib
 import multiprocessing as mp
 import os
 import pickle
@@ -41,26 +40,13 @@ def cpu_model() -> str:
     return "unknown"
 
 
-def build_perf(verbose: bool = False) -> str:
-    """-O3 -march=native copy of the oracle for TIMING (oracle/_perf/libicg_oracle_perf_<cpu-flags hash>.so), built where it runs."""
-    flags = ""
-    try:
-        for line in open("/proc/cpuinfo"):
-            if line.startswith("flags"):
-                flags = line
-                break
-    except OSError:
-        pass
-    tag = hashlib.sha1(flags.encode()).hexdigest()[:10]
-    out_dir = os.path.join(HERE, "_perf")
-    os.makedirs(out_dir, exist_ok=True)
-    out = os.path.join(out_dir, f"libicg_oracle_perf_{tag}.so")
+def build_perf(out_dir: str, verbose: bool = False) -> str:
+    """-O3 -march=native copy of the oracle for TIMING (<out_dir>/libicg_oracle_perf.so), built where it runs."""
+    out = os.path.join(out_dir, "libicg_oracle_perf.so")
     srcs = [os.path.join(HERE, f) for f in ("klt_ref.c", "detect_ref.c", "clahe_ref.c", "ba_ref.cpp")]
-    if os.path.exists(out) and all(os.path.getmtime(out) >= os.path.getmtime(s) for s in srcs + [os.path.join(HERE, "ba_ref.hpp")]):
-        return out
     objs = []
     for s in srcs:
-        o = os.path.join(out_dir, os.path.basename(s) + f".{tag}.o")
+        o = os.path.join(out_dir, os.path.basename(s) + ".o")
         cc = ["g++", "-std=c++17", "-pthread"] if s.endswith(".cpp") else ["gcc", "-std=c11"]
         cmd = cc + ["-O3", "-march=native", "-fPIC", "-fno-fast-math", "-c", s, "-o", o]
         if verbose:
@@ -142,11 +128,17 @@ def measure(frames, pairs, probs, reps=5, n_frames=8, do_ba=True, max_procs=None
     cores = sorted(os.sched_getaffinity(0))
     if max_procs:
         cores = cores[:max_procs]
+    with tempfile.TemporaryDirectory(prefix="icg_cpu_arm_") as td:
+        perf_so = build_perf(td)
+        path = os.path.join(td, "inputs.pkl")
+        with open(path, "wb") as f:
+            pickle.dump(dict(frames=frames, pairs=pairs, probs=probs if do_ba else []), f, protocol=pickle.HIGHEST_PROTOCOL)
+        return _measure(cores, perf_so, path, reps, n_frames, do_ba)
+
+
+def _measure(cores, perf_so, path, reps, n_frames, do_ba):
+    """one pinned worker per core; `perf_so` and the pickled inputs at `path` live in measure()'s temporary directory"""
     nproc = len(cores)
-    perf_so = build_perf()
-    fd, path = tempfile.mkstemp(suffix=".pkl", prefix="icg_cpu_arm_")
-    with os.fdopen(fd, "wb") as f:
-        pickle.dump(dict(frames=frames, pairs=pairs, probs=probs if do_ba else []), f, protocol=pickle.HIGHEST_PROTOCOL)
     ctx = mp.get_context("spawn")
     barrier, q = ctx.Barrier(nproc), ctx.Queue()
     load0 = os.getloadavg()
@@ -169,10 +161,6 @@ def measure(frames, pairs, probs, reps=5, n_frames=8, do_ba=True, max_procs=None
             p.join(30)
             if p.is_alive():
                 p.kill()
-        try:
-            os.unlink(path)
-        except OSError:
-            pass
     per_rep, klt_rep, ba_rep = [], [], []
     for r in range(reps):
         rr = [x for x in rows if x[1] == r]

@@ -1,6 +1,8 @@
 """Generates tests/golden/clahe_golden.npz with cv2 (the OpenCV the reference links): `cv::createCLAHE(3.0, Size(21, 21))->apply(img, img)`
-exactly as ic_gvins/ic_gvins/tracking/tracking.cc:62,141 calls it, plus parameter / size variations.  Run in the build container
-(cv2 4.13.0); the GPU box never imports cv2 for the parity tests."""
+exactly as ic_gvins/ic_gvins/tracking/tracking.cc:62,141 calls it, plus parameter / size variations.  Needs cv2 (the stored file
+was made with 4.13.0); the parity tests never import it.  Each case keeps its input image and the SHA-256 of cv2's uint8 output:
+the textured images barely compress, and the full outputs would more than double the file."""
+import hashlib
 import os
 
 import cv2
@@ -32,7 +34,7 @@ def main():
             img[:30] = 17  # a flat half: exercises clipping + residual redistribution
         ref = cv2.createCLAHE(clip, (tx, ty)).apply(img)
         out[name + "_in"] = img
-        out[name + "_out"] = ref
+        out[name + "_out_sha256"] = hashlib.sha256(ref.tobytes()).hexdigest()
         out[name + "_par"] = np.array([tx, ty, clip], np.float64)
     np.savez_compressed(os.path.join(HERE, "clahe_golden.npz"), cv2_version=cv2.__version__, **out)
     print("wrote clahe_golden.npz:", list(spec))
