@@ -40,6 +40,24 @@ class BaPrior(C.Structure):
                 ("x0", dp), ("J0", dp), ("e0", dp), ("Hp", dp), ("bp", dp)]
 
 
+class Camera(C.Structure):
+    """ctypes image of `icg_camera`."""
+    _fields_ = [(k, C.c_double) for k in ("fx", "fy", "cx", "cy", "skew", "k1", "k2", "p1", "p2", "k3")]
+
+
+class CullInput(C.Structure):
+    """ctypes image of `icg_ba_cull_input`."""
+    _fields_ = [("cam", Camera), ("reprojection_error_std", C.c_double), ("estimate_extrinsic", C.c_int32), ("reserved", C.c_int32),
+                ("R_bc", C.c_double * 9), ("t_bc", C.c_double * 3), ("f_kp", C.POINTER(C.c_float)), ("lm_ref_kp", C.POINTER(C.c_float)),
+                ("lm_ref_node", ip), ("lm_ref_pos", ip)]
+
+
+class CullOutput(C.Structure):
+    """ctypes image of `icg_ba_cull_output`."""
+    _fields_ = [("ext_updated", C.c_int32), ("counts", C.c_int32 * 5), ("R_bc", C.c_double * 9), ("t_bc", C.c_double * 3),
+                ("cam_pose", dp), ("lm_pos", dp), ("lm_depth", dp), ("f_outlier", bp), ("lm_ref_outlier", bp), ("lm_outlier", bp)]
+
+
 class BaSummary(C.Structure):
     _fields_ = [("iterations", C.c_int32), ("num_successful_steps", C.c_int32), ("termination", C.c_int32), ("reserved", C.c_int32),
                 ("initial_cost", C.c_double), ("final_cost", C.c_double), ("final_radius", C.c_double)]
@@ -259,6 +277,43 @@ class WindowSolver:
         call = self.marg_prepare(problems, num_marg, want_schur)
         self.marg_run(call, resident)
         return self.marg_collect(call)
+
+    def outlier_culling(self, problems, cull_inputs, want_geometry=True):
+        """GVINS::updateParametersFromOptimizer + gvinsOutlierCulling (IG/ic_gvins.cc:1299-1389, 1035-1128) on the windows this handle has just
+        solved (icg_ba_outlier_culling_resident; `problems` = the list of that solve).  cull_inputs: one dict per window with `cam` (fx, fy, cx,
+        cy[, skew]), `reprojection_error_std` (px), `estimate_extrinsic`, `R_bc` (3x3), `t_bc`, `f_kp` (F x 2), `lm_ref_kp` (L x 2),
+        `lm_ref_node`, `lm_ref_pos` (L).  Each problem's f_active becomes the culling mask (in place).  Returns one dict per window: ext_updated,
+        R_bc, t_bc, counts (outliers_[0], outliers_[1], num1, num2, num3), f_outlier, lm_ref_outlier, lm_outlier (bits num1 | num2 << 1 | num3 << 2)
+        and, with want_geometry, cam_pose (K x 12: R_wc row-major, t_wc), lm_pos (L x 3), lm_depth."""
+        if isinstance(problems, dict):
+            problems, cull_inputs = [problems], [cull_inputs]
+        n = len(problems)
+        arr = (BaProblem * n)(*[to_struct(p) for p in problems])
+        cin, cout = (CullInput * n)(), (CullOutput * n)()
+        keep, res = [], []
+        for w, (p, c) in enumerate(zip(problems, cull_inputs)):
+            cam = list(c["cam"]) + [0.0] * (10 - len(c["cam"]))
+            cin[w].cam = Camera(*[float(x) for x in cam])
+            cin[w].reprojection_error_std = float(c["reprojection_error_std"])
+            cin[w].estimate_extrinsic = int(bool(c["estimate_extrinsic"]))
+            cin[w].R_bc[:] = [float(x) for x in np.asarray(c["R_bc"], np.float64).ravel()]
+            cin[w].t_bc[:] = [float(x) for x in np.asarray(c["t_bc"], np.float64).ravel()]
+            dts = dict(f_kp=np.float32, lm_ref_kp=np.float32, lm_ref_node=np.int32, lm_ref_pos=np.int32)
+            a = {k: np.ascontiguousarray(c[k], dt) for k, dt in dts.items() if c[k] is not None}  # None passes NULL (argument checks)
+            o = dict(f_outlier=np.zeros(p["F"], np.uint8), lm_ref_outlier=np.zeros(p["L"], np.uint8), lm_outlier=np.zeros(p["L"], np.uint8))
+            if want_geometry:
+                o.update(cam_pose=np.zeros((p["K"], 12)), lm_pos=np.zeros((p["L"], 3)), lm_depth=np.zeros(p["L"]))
+            for k, v in a.items():
+                setattr(cin[w], k, v.ctypes.data_as(C.POINTER(C.c_float) if v.dtype == np.float32 else ip) if v.size else None)
+            for k, v in o.items():
+                setattr(cout[w], k, v.ctypes.data_as(dp if v.dtype == np.float64 else bp) if v.size else None)
+            keep.append(a)
+            res.append(o)
+        check(lib().icg_ba_outlier_culling_resident(self._h, n, arr, cin, cout), "icg_ba_outlier_culling_resident")
+        for w, o in enumerate(res):
+            o.update(ext_updated=int(cout[w].ext_updated), counts=np.array(cout[w].counts[:], np.int32),
+                     R_bc=np.array(cout[w].R_bc[:]).reshape(3, 3), t_bc=np.array(cout[w].t_bc[:]))
+        return res
 
     def marg_prepare(self, problems, num_marg=1, want_schur=True):
         """The argument block of one icg_ba_marginalize call (struct array over the problems' host arrays + caller-allocated output arrays):

@@ -26,6 +26,7 @@ SOURCES = {
     "fundamental.cu": ["-fmad=false"],  # host code; no contraction of the reference's double sequence
     "geom.cu": ["-fmad=false"],         # device versions of the camera model / RANSAC gate / triangulation / IMU propagation (same cores)
     "ba.cu": [],
+    "ba_cull.cu": ["-fmad=false"],      # post-solve outlier culling: the float cast in cam2pixel makes its decisions sensitive to contraction
 }
 
 

@@ -33,6 +33,7 @@
 #include <thread>
 #include <vector>
 
+#include "ba_cull.cuh"
 #include "ba_math.cuh"
 #include "common.cuh"
 #include "geom_core.cuh"
@@ -1818,6 +1819,8 @@ struct icg_ba {
     MargDev M;
     HostDev<int> marg_map;
     HostDev<double> marg_oJ0, marg_oe0, marg_oHp, marg_obp;
+    // outlier-culling staging buffer (ba_cull.cuh layout; allocated on the first icg_ba_outlier_culling_resident call)
+    HostDev<unsigned char> cull_buf;
 };
 
 extern "C" {
@@ -2036,6 +2039,7 @@ void icg_ba_destroy(icg_ba *h) {
     if (h->comm) nccl_api().CommDestroy((ncclComm_t) h->comm);
     split_release(h);
     if (h->marg_ready) h->marg_map.release(), h->marg_oJ0.release(), h->marg_oe0.release(), h->marg_oHp.release(), h->marg_obp.release();
+    h->cull_buf.release();
     for (void *p : h->dev_only) cudaFree(p);
     if (h->stream_cam) cudaStreamSynchronize(h->stream_cam), cudaStreamDestroy(h->stream_cam);
     if (h->ev_fork) cudaEventDestroy(h->ev_fork);
@@ -2918,6 +2922,142 @@ int icg_ba_marginalize(icg_ba *h, int n_windows, const icg_ba_problem *problems,
 
 int icg_ba_marginalize_resident(icg_ba *h, int n_windows, const icg_ba_problem *problems, const int32_t *num_marg, icg_ba_prior *out) {
     return marginalize_body(h, n_windows, problems, num_marg, out, true);
+}
+
+// ---- post-solve outlier culling (updateParametersFromOptimizer + gvinsOutlierCulling, kernel in ba_cull.cu)
+static size_t cull_layout(int n, size_t Ft, size_t Lt, size_t Kt, CullLaunch &A) {  // byte offsets of the sections (ba_cull.cuh); returns the end
+    auto al = [](size_t x) { return (x + 15) & ~(size_t) 15; };
+    size_t o = 0;
+    A.o_win = o, o = al(o + n * sizeof(CullWin));
+    A.o_fkp = o, o = al(o + Ft * 2 * sizeof(float));
+    A.o_lkp = o, o = al(o + Lt * 2 * sizeof(float));
+    A.o_lnode = o, o = al(o + Lt * sizeof(int));
+    A.o_lpos = o, o = al(o + Lt * sizeof(int));
+    A.o_wout = o, o = al(o + n * sizeof(CullWinOut));
+    A.o_fout = o, o = al(o + Ft);
+    A.o_lrout = o, o = al(o + Lt);
+    A.o_lout = o, o = al(o + Lt);
+    A.o_cam = o, o = al(o + Kt * 12 * sizeof(double));
+    A.o_depth = o, o = al(o + Lt * sizeof(double));
+    A.o_pos = o, o = al(o + Lt * 3 * sizeof(double));
+    return o;
+}
+
+int icg_ba_outlier_culling_resident(icg_ba *h, int n_windows, const icg_ba_problem *problems, const icg_ba_cull_input *in, icg_ba_cull_output *out) {
+    if (!h || !problems || !in || !out || n_windows < 1) {
+        set_error("icg_ba_outlier_culling_resident: bad arguments");
+        return ICG_EINVAL;
+    }
+    if (h->comm || h->D.world > 1) {
+        set_error("icg_ba_outlier_culling_resident: not available on a landmark-sharded handle (icg_ba_set_shard(world = 1) first)");
+        return ICG_EUNSUPPORTED;
+    }
+    if (h->cur_windows != n_windows) {
+        set_error("icg_ba_outlier_culling_resident: the handle holds %d uploaded windows, the call names %d", h->cur_windows, n_windows);
+        return ICG_EINVAL;
+    }
+    const BaCaps &C = h->C;
+    const int n = n_windows;
+    // ---- argument checks (nothing is launched on failure)
+    size_t Ft = 0, Lt = 0, Kt = 0;
+    int max_L = 0;
+    for (int w = 0; w < n; w++) {
+        const icg_ba_problem &p = problems[w];
+        const icg_ba_cull_input &c = in[w];
+        const icg_ba_cull_output &o = out[w];
+        const WinDims &d = h->dims.h[w];
+        if (p.K != d.K || p.L != d.L || p.F != d.F) {
+            set_error("icg_ba_outlier_culling_resident: window %d is not the uploaded one (K=%d L=%d F=%d, uploaded %d %d %d)", w, p.K, p.L, p.F, d.K, d.L, d.F);
+            return ICG_EINVAL;
+        }
+        if ((p.F > 0 && (!p.f_lm || !p.f_ref || !p.f_active || !c.f_kp || !o.f_outlier)) ||
+            (p.L > 0 && (!c.lm_ref_kp || !c.lm_ref_node || !c.lm_ref_pos || !o.lm_ref_outlier || !o.lm_outlier)) || !(c.reprojection_error_std > 0)) {
+            set_error("icg_ba_outlier_culling_resident: window %d: a required array is NULL or reprojection_error_std <= 0", w);
+            return ICG_EINVAL;
+        }
+        const int *off = h->lm_off.h + (size_t) w * (C.L + 1);
+        for (int l = 0; l < p.L; l++) {
+            if (c.lm_ref_node[l] < 0 || c.lm_ref_node[l] >= p.K || c.lm_ref_pos[l] < 0 || c.lm_ref_pos[l] > off[l + 1] - off[l]) {
+                set_error("icg_ba_outlier_culling_resident: window %d landmark %d: lm_ref_node %d / lm_ref_pos %d out of range (%d factors)", w, l, c.lm_ref_node[l],
+                          c.lm_ref_pos[l], off[l + 1] - off[l]);
+                return ICG_EINVAL;
+            }
+        }
+        for (int f = 0; f < p.F; f++) {
+            if (p.f_ref[f] != c.lm_ref_node[p.f_lm[f]]) {
+                set_error("icg_ba_outlier_culling_resident: window %d factor %d: f_ref %d differs from the landmark's reference node %d", w, f, p.f_ref[f],
+                          c.lm_ref_node[p.f_lm[f]]);
+                return ICG_EINVAL;
+            }
+        }
+        Ft += p.F, Lt += p.L, Kt += p.K, max_L = std::max(max_L, p.L);
+    }
+    ICG_CUDA(cudaSetDevice(h->device));
+    CullLaunch A;
+    if (!h->cull_buf.h) {
+        const size_t cap = cull_layout(C.NW, (size_t) C.NW * C.F, (size_t) C.NW * C.L, (size_t) C.NW * C.K, A);
+        if (h->cull_buf.alloc(cap) != ICG_OK) {
+            h->cull_buf.release();
+            set_error("icg_ba_outlier_culling_resident: staging allocation failed");
+            return ICG_ENOMEM;
+        }
+    }
+    const size_t end = cull_layout(n, Ft, Lt, Kt, A);
+    // ---- pack the inputs (+ zeroed per-window output records: the counters start at zero)
+    unsigned char *hb = h->cull_buf.h;
+    {
+        size_t f0 = 0, l0 = 0, k0 = 0;
+        for (int w = 0; w < n; w++) {
+            const icg_ba_problem &p = problems[w];
+            const icg_ba_cull_input &c = in[w];
+            CullWin &W = ((CullWin *) (hb + A.o_win))[w];
+            W.cam = c.cam, W.reproj_std = c.reprojection_error_std;
+            memcpy(W.R_bc, c.R_bc, sizeof(W.R_bc)), memcpy(W.t_bc, c.t_bc, sizeof(W.t_bc));
+            W.estimate_extrinsic = c.estimate_extrinsic != 0, W.K = p.K, W.L = p.L, W.F = p.F;
+            W.f0 = (int) f0, W.l0 = (int) l0, W.k0 = (int) k0, W.pad = 0;
+            if (p.F) memcpy(hb + A.o_fkp + f0 * 8, c.f_kp, (size_t) p.F * 8);
+            if (p.L) {
+                memcpy(hb + A.o_lkp + l0 * 8, c.lm_ref_kp, (size_t) p.L * 8);
+                memcpy(hb + A.o_lnode + l0 * 4, c.lm_ref_node, (size_t) p.L * 4);
+                memcpy(hb + A.o_lpos + l0 * 4, c.lm_ref_pos, (size_t) p.L * 4);
+            }
+            f0 += p.F, l0 += p.L, k0 += p.K;
+        }
+        memset(hb + A.o_wout, 0, n * sizeof(CullWinOut));
+    }
+    const BaDev &D = h->D;
+    A.pose = D.pose, A.ext = D.ext, A.rho = D.rho, A.lm_off = D.lm_off, A.f_meta_s = D.f_meta_s, A.f_active = D.f_active;
+    A.capK = C.K, A.capL = C.L, A.capF = C.F, A.buf = h->cull_buf.d;
+    size_t d2h_end = A.o_cam;  // the D2H stops after the last section some window asked for
+    for (int w = 0; w < n; w++) {
+        if (out[w].lm_pos) d2h_end = std::max(d2h_end, end);
+        else if (out[w].lm_depth) d2h_end = std::max(d2h_end, A.o_pos);
+        else if (out[w].cam_pose) d2h_end = std::max(d2h_end, A.o_depth);
+    }
+    cudaStream_t s = h->stream;
+    ICG_CUDA(cudaMemcpyAsync(h->cull_buf.d, hb, A.o_wout + n * sizeof(CullWinOut), cudaMemcpyHostToDevice, s));
+    ICG_CUDA(launch_outlier_cull(A, n, max_L, s));
+    ICG_CUDA(cudaMemcpyAsync(hb + A.o_wout, h->cull_buf.d + A.o_wout, d2h_end - A.o_wout, cudaMemcpyDeviceToHost, s));
+    ICG_CUDA(cudaStreamSynchronize(s));
+    // ---- results into the caller's arrays; f_active of the problems mirrors the device copy
+    size_t f0 = 0, l0 = 0, k0 = 0;
+    for (int w = 0; w < n; w++) {
+        const icg_ba_problem &p = problems[w];
+        icg_ba_cull_output &o = out[w];
+        const CullWinOut &WO = ((const CullWinOut *) (hb + A.o_wout))[w];
+        o.ext_updated = WO.ext_updated;
+        memcpy(o.counts, WO.counts, sizeof(o.counts)), memcpy(o.R_bc, WO.R_bc, sizeof(o.R_bc)), memcpy(o.t_bc, WO.t_bc, sizeof(o.t_bc));
+        const uint8_t *fo = hb + A.o_fout + f0, *lo = hb + A.o_lout + l0;
+        if (p.F) memcpy(o.f_outlier, fo, p.F);
+        if (p.L) memcpy(o.lm_ref_outlier, hb + A.o_lrout + l0, p.L), memcpy(o.lm_outlier, lo, p.L);
+        if (o.cam_pose) memcpy(o.cam_pose, hb + A.o_cam + k0 * 96, (size_t) p.K * 96);
+        if (o.lm_depth && p.L) memcpy(o.lm_depth, hb + A.o_depth + l0 * 8, (size_t) p.L * 8);
+        if (o.lm_pos && p.L) memcpy(o.lm_pos, hb + A.o_pos + l0 * 24, (size_t) p.L * 24);
+        uint8_t *act = const_cast<uint8_t *>(p.f_active);
+        for (int f = 0; f < p.F; f++) act[f] = (uint8_t) (!fo[f] && !lo[p.f_lm[f]]);
+        f0 += p.F, l0 += p.L, k0 += p.K;
+    }
+    return ICG_OK;
 }
 
 int icg_nccl_unique_id(uint8_t *id128) {

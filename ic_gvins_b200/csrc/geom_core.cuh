@@ -421,5 +421,94 @@ GC_HD void preintegrate_core(const double *state16, const double *iewn3, const d
     }
 }
 
+// ------------------------------------------------------------------------------------------------ post-solve update + outlier culling
+// GVINS::updateParametersFromOptimizer (IG/ic_gvins.cc:1299-1389) and the per-observation test of GVINS::gvinsOutlierCulling (:1035-1128).
+// Written out operation by operation (no library products) so that host, device and a plain scalar restatement
+// round alike; the device copy is compiled without FMA contraction (the float cast in cam2pixel makes the decisions sensitive to it).
+// Eigen's Quaternion::normalized(): coeffs (x, y, z, w) / sqrt(squaredNorm), squared norm summed in storage order
+GC_HD bam::Q quat_normalized(bam::Q q) {
+    const double n = sqrt(((q.x * q.x + q.y * q.y) + q.z * q.z) + q.w * q.w);
+    return bam::mkq(q.w / n, q.x / n, q.y / n, q.z / n);
+}
+// Eigen's Quaternion(const Matrix3 &) (quaternionbase_assign_impl<Other, 3, 3>), row-major R
+GC_HD bam::Q rot_to_quat(const double *R) {
+    bam::Q q;
+    double t = (R[0] + R[4]) + R[8];
+    if (t > 0.0) {
+        t = sqrt(t + 1.0);
+        q.w = 0.5 * t;
+        t = 0.5 / t;
+        q.x = (R[7] - R[5]) * t;
+        q.y = (R[2] - R[6]) * t;
+        q.z = (R[3] - R[1]) * t;
+    } else {
+        int i = 0;
+        if (R[4] > R[0]) i = 1;
+        if (R[8] > R[3 * i + i]) i = 2;
+        const int j = (i + 1) % 3, k = (j + 1) % 3;
+        double c[3];
+        t = sqrt(((R[3 * i + i] - R[3 * j + j]) - R[3 * k + k]) + 1.0);
+        c[i] = 0.5 * t;
+        t = 0.5 / t;
+        q.w = (R[3 * k + j] - R[3 * j + k]) * t;
+        c[j] = (R[3 * j + i] + R[3 * i + j]) * t;
+        c[k] = (R[3 * k + i] + R[3 * i + k]) * t;
+        q.x = c[0], q.y = c[1], q.z = c[2];
+    }
+    return q;
+}
+// the extrinsic gate of updateParametersFromOptimizer (:1311-1331): candidate (t, R) from ext = (t, q_xyzw, td), accepted unless
+// |t - t_bc| > 1 m or |vec(quaternion(R R_bc^T))| * R2D > 5 (sin(theta / 2) in "degrees": the gate trips near theta = 10 deg, as written).
+// R_bc / t_bc are updated in place; returns 1 when the candidate was taken.
+GC_HD int extrinsic_gate(const double *ext, double *R_bc, double *t_bc) {
+    const bam::Q q = quat_normalized(bam::mkq(ext[6], ext[3], ext[4], ext[5]));
+    const bam::M3 R = bam::qmat(q);
+    const double dx = ext[0] - t_bc[0], dy = ext[1] - t_bc[1], dz = ext[2] - t_bc[2];
+    const double dt = sqrt((dx * dx + dy * dy) + dz * dz);
+    bam::M3 Rb;
+    for (int i = 0; i < 9; i++) Rb.m[i] = R_bc[i];
+    const bam::M3 D = bam::mul(R, bam::tr(Rb));
+    const bam::Q qd = rot_to_quat(D.m);
+    const double dr = sqrt((qd.x * qd.x + qd.y * qd.y) + qd.z * qd.z) * (180.0 / 3.14159265358979323846);
+    if (dt > 1.0 || dr > 5.0) return 0;
+    for (int i = 0; i < 9; i++) R_bc[i] = R.m[i];
+    for (int i = 0; i < 3; i++) t_bc[i] = ext[i];
+    return 1;
+}
+// MISC::stateToCameraPose (IG/misc.cc:102-108) of a node pose7 = (p, q_xyzw): R_wc = R(q) R_bc, t_wc = p + R(q) t_bc (q normalised first,
+// PreintegrationBase::stateFromData, preintegration_base.cc:115-125)
+GC_HD void camera_pose(const double *pose7, const double *R_bc, const double *t_bc, double *R_wc, double *t_wc) {
+    const bam::M3 Rq = bam::qmat(quat_normalized(bam::mkq(pose7[6], pose7[3], pose7[4], pose7[5])));
+    bam::M3 Rb;
+    for (int i = 0; i < 9; i++) Rb.m[i] = R_bc[i];
+    const bam::M3 Rw = bam::mul(Rq, Rb);
+    const bam::V3 rt = bam::mul(Rq, bam::mk(t_bc[0], t_bc[1], t_bc[2]));
+    for (int i = 0; i < 9; i++) R_wc[i] = Rw.m[i];
+    t_wc[0] = pose7[0] + rt.x, t_wc[1] = pose7[1] + rt.y, t_wc[2] = pose7[2] + rt.z;
+}
+// map point from its reference key point and inverse depth (:1379-1386): pos = R_ref (pixel2cam(kp) * depth) + t_ref, depth = 1 / invdepth
+GC_HD void mappoint_position(const icg_camera &c, const double *R_ref, const double *t_ref, float ku, float kv, double invdepth, double *pos, double &depth) {
+    depth = 1.0 / invdepth;
+    double x, y;
+    pixel2cam(c, ku, kv, x, y);
+    const bam::V3 pw = bam::mul(*(const bam::M3 *) R_ref, bam::mk(x * depth, y * depth, 1.0 * depth));
+    pos[0] = pw.x + t_ref[0], pos[1] = pw.y + t_ref[1], pos[2] = pw.z + t_ref[2];
+}
+// Tracking::isGoodToTrack(kp, pose, pos, scale) (IG/tracking/tracking.cc:813-828): depth gate 1 < z_c < 200 (isGoodDepth, :247-249) and the
+// reprojection error |world2pixel(pos) - kp| (Camera::reprojectionError, camera.cc:153-157: float difference, double norm) <= threshold.
+// err receives that error; it is what gvinsOutlierCulling averages (:1075).
+GC_HD bool good_to_track(const icg_camera &c, const double *R_wc, const double *t_wc, const double *pos, float ku, float kv, double threshold, double &err) {
+    const double vx = pos[0] - t_wc[0], vy = pos[1] - t_wc[1], vz = pos[2] - t_wc[2];
+    const double pcx = (R_wc[0] * vx + R_wc[3] * vy) + R_wc[6] * vz;  // R^T (pw - t)
+    const double pcy = (R_wc[1] * vx + R_wc[4] * vy) + R_wc[7] * vz;
+    const double pcz = (R_wc[2] * vx + R_wc[5] * vy) + R_wc[8] * vz;
+    float u, v;
+    cam2pixel(c, pcx, pcy, pcz, u, v);
+    const double ex = (double) (u - ku), ey = (double) (v - kv);
+    err = sqrt(ex * ex + ey * ey);
+    if (!(pcz > 1.0 && pcz < 200.0)) return false;
+    return !(err > threshold);
+}
+
 }  // namespace gc
 }  // namespace icg

@@ -138,6 +138,25 @@ public:
         return P;
     }
 
+    // updateParametersFromOptimizer() + gvinsOutlierCulling() (IG/ic_gvins.cc:1232-1236): the culling verdicts of the window this solver has
+    // just optimised (after_solve; otherwise the problem is uploaded first and culled at its own parameters).  problem.f_active becomes the mask
+    // gvinsMarginalization finds in the map; the caller removes the flagged map points (Map::removeMappoint) and sets pose_b_c_ = R_bc, t_bc.
+    struct Culling {
+        icg_ba_cull_output out{};                           // ext_updated, counts, R_bc, t_bc
+        std::vector<uint8_t> f_outlier, lm_ref_outlier, lm_outlier;
+        std::vector<double> cam_pose, lm_pos, lm_depth;     // K x 12, L x 3, L
+    };
+    Culling outlierCulling(const icg_ba_problem &problem, const icg_ba_cull_input &in, bool after_solve = true) {
+        Culling C;
+        C.f_outlier.resize(problem.F), C.lm_ref_outlier.resize(problem.L), C.lm_outlier.resize(problem.L);
+        C.cam_pose.resize((size_t) problem.K * 12), C.lm_pos.resize((size_t) problem.L * 3), C.lm_depth.resize(problem.L);
+        C.out.f_outlier = C.f_outlier.data(), C.out.lm_ref_outlier = C.lm_ref_outlier.data(), C.out.lm_outlier = C.lm_outlier.data();
+        C.out.cam_pose = C.cam_pose.data(), C.out.lm_pos = C.lm_pos.data(), C.out.lm_depth = C.lm_depth.data();
+        if (!after_solve) check(icg_ba_upload(h_, 1, &problem), "icg_ba_upload");
+        check(icg_ba_outlier_culling_resident(h_, 1, &problem, &in, &C.out), "icg_ba_outlier_culling_resident");
+        return C;
+    }
+
 private:
     icg_ba *h_ = nullptr;
 };

@@ -343,6 +343,47 @@ int icg_ba_marginalize(icg_ba *h, int n_windows, const icg_ba_problem *problems,
  * of that solve (n_windows equal to the uploaded count; read for the factor structure and x0 only). */
 int icg_ba_marginalize_resident(icg_ba *h, int n_windows, const icg_ba_problem *problems, const int32_t *num_marg, icg_ba_prior *out);
 /*
+ * The end of GVINS::gvinsOptimization on the windows the handle holds: updateParametersFromOptimizer (IG/ic_gvins.cc:1299-1389) and
+ * gvinsOutlierCulling (:1035-1128), in one launch over the batch.  Per window:
+ *   1. extrinsic gate (only with estimate_extrinsic): the solved extrinsic replaces (R_bc, t_bc) unless |dt| > 1 m or
+ *      |vec(quaternion(R R_bc^T))| * 180 / pi > 5 (sin(theta / 2) in "degrees", as the reference writes it);
+ *   2. camera pose of every node, MISC::stateToCameraPose (IG/misc.cc:102-108), with the gated extrinsic;
+ *   3. map point of every landmark: R_ref (pixel2cam(lm_ref_kp) / invdepth) + t_ref;
+ *   4. every observation in mappoint->observations() order -- the reference observation at position lm_ref_pos, the landmark's factors in
+ *      ascending factor index around it (the order addReprojectionFactors creates them in, :1777-1834) -- through
+ *      Tracking::isGoodToTrack(kp, pose, pos, 3.0) (1 < z_c < 200, |world2pixel - kp| <= 3 std): a bad one is a feature outlier; a bad
+ *      reference observation makes the landmark an outlier (num1) and ends its loop; then fewer than 2 good errors (num2) or a mean error
+ *      above std (num3) makes it an outlier.  f_active is ignored: every factor of the window is evaluated.
+ * Afterwards f_active[f] = !f_outlier[f] && !lm_outlier[f_lm[f]] on the device and in problems[w].f_active (updated in place, as
+ * icg_ba_gvins_optimization does), so icg_ba_marginalize_resident builds the prior from the factors gvinsMarginalization finds in the map
+ * (:1559-1590).  Removing the map points (Map::removeMappoint) stays with the caller.  `problems` must be the array of the last upload
+ * (n_windows equal to the uploaded count); it is read for f_lm / f_ref and written through f_active only.
+ * Errors: ICG_EINVAL when a required array is NULL, f_ref[f] != lm_ref_node[f_lm[f]], lm_ref_pos is outside [0, factors of the landmark]
+ * or n_windows differs from the uploaded count (nothing is launched); ICG_EUNSUPPORTED on a landmark-sharded handle.
+ */
+typedef struct icg_ba_cull_input {
+    icg_camera cam;                /* pinhole part only: fx, fy, cx, cy, skew (Camera::world2pixel, IG/tracking/camera.cc:129-146) */
+    double reprojection_error_std; /* pixels (IG/ic_gvins.cc:133) */
+    int32_t estimate_extrinsic;    /* optimize_estimate_extrinsic_ */
+    int32_t reserved;
+    double R_bc[9], t_bc[3];       /* pose_b_c_ before the call (R row-major): the gate's baseline */
+    const float *f_kp;             /* F x 2: keyPoint() of each factor's observing feature */
+    const float *lm_ref_kp;        /* L x 2: referenceKeypoint() */
+    const int32_t *lm_ref_node;    /* L: reference node (a landmark may have no factor) */
+    const int32_t *lm_ref_pos;     /* L: position of the reference observation in observations(), 0 .. factors of the landmark */
+} icg_ba_cull_input;
+typedef struct icg_ba_cull_output {
+    int32_t ext_updated;           /* 1: pose_b_c_ took the solved extrinsic */
+    int32_t counts[5];             /* outliers_[0] (map-point outliers, num1 + (num2 or num3)), outliers_[1] (feature outliers), num1, num2, num3 */
+    double R_bc[9], t_bc[3];       /* pose_b_c_ after the gate */
+    double *cam_pose;              /* K x 12 (R_wc row-major, t_wc), may be NULL */
+    double *lm_pos, *lm_depth;     /* L x 3 and L, may be NULL */
+    uint8_t *f_outlier;            /* F: feature outlier (setOutlier on the observing feature) */
+    uint8_t *lm_ref_outlier;       /* L: the reference observation was flagged */
+    uint8_t *lm_outlier;           /* L: bit 0 num1, bit 1 num2, bit 2 num3 */
+} icg_ba_cull_output;
+int icg_ba_outlier_culling_resident(icg_ba *h, int n_windows, const icg_ba_problem *problems, const icg_ba_cull_input *in, icg_ba_cull_output *out);
+/*
  * Landmark sharding of the window solve across the GPUs of one box (SURVEY.md 8e): every process (one per GPU) uploads the same
  * camera-side problem but only ITS landmarks and their reprojection factors; per LM attempt one NCCL sum all-reduce of the packed
  * [vision Gram matrix + gradient | Schur term | vision cost, sum rho^2] buffer (+ an n-double max / 4n-double sum) makes the
