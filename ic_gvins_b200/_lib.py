@@ -96,8 +96,6 @@ def _declare(L: C.CDLL) -> None:
     L.icg_ba_run.argtypes = [vp, C.c_int, C.c_int]
     L.icg_ba_download.argtypes = [vp, C.c_int, vp, vp]
     L.icg_ba_sync.argtypes = [vp]
-    L.icg_nccl_unique_id.argtypes = [vp]
-    L.icg_ba_set_shard.argtypes = [vp, C.c_int, C.c_int, vp]
     L.icg_ba_shard_export.argtypes = [vp, C.c_int, C.c_int, vp]
     L.icg_ba_shard_connect.argtypes = [vp, vp]
     L.icg_ba_shard_error.argtypes = [vp]
@@ -140,5 +138,5 @@ EXPORTS = [
     "icg_camera_undistort_points", "icg_camera_distort_points", "icg_camera_distort_camera_points", "icg_camera_pixel2cam", "icg_camera_world2pixel", "icg_tracking_histogram", "icg_find_fundamental_mat_ransac", "icg_triangulate_points",
     "icg_clahe_create", "icg_clahe_destroy", "icg_clahe_apply", "icg_clahe_apply_dev", "icg_clahe_apply_batch_dev", "icg_geom_create", "icg_geom_destroy", "icg_geom_undistort_points", "icg_geom_distort_points", "icg_geom_find_fundamental_mat_ransac", "icg_geom_triangulate_points", "icg_geom_imu_preintegrate_batch", "icg_clahe_sync",
     "icg_imu_preintegrate", "icg_ba_create", "icg_ba_destroy", "icg_ba_solve", "icg_ba_upload", "icg_ba_run", "icg_ba_download",
-    "icg_ba_sync", "icg_nccl_unique_id", "icg_ba_set_shard", "icg_ba_shard_export", "icg_ba_shard_connect", "icg_ba_shard_error", "icg_ba_gvins_optimization", "icg_ba_run_gvins", "icg_ba_gvins_optimization_begin", "icg_ba_gvins_optimization_end", "icg_ba_residual_costs", "icg_ba_reproj_evaluate", "icg_ba_imu_evaluate", "icg_ba_marginalize", "icg_ba_marginalize_resident", "icg_ba_outlier_culling_resident", "icg_ba_gnss_evaluate", "icg_ba_pose_prior_evaluate", "icg_ba_mix_prior_evaluate", "icg_ba_imu_error_evaluate", "icg_ba_marg_factor_evaluate",
+    "icg_ba_sync", "icg_ba_shard_export", "icg_ba_shard_connect", "icg_ba_shard_error", "icg_ba_gvins_optimization", "icg_ba_run_gvins", "icg_ba_gvins_optimization_begin", "icg_ba_gvins_optimization_end", "icg_ba_residual_costs", "icg_ba_reproj_evaluate", "icg_ba_imu_evaluate", "icg_ba_marginalize", "icg_ba_marginalize_resident", "icg_ba_outlier_culling_resident", "icg_ba_gnss_evaluate", "icg_ba_pose_prior_evaluate", "icg_ba_mix_prior_evaluate", "icg_ba_imu_error_evaluate", "icg_ba_marg_factor_evaluate",
 ]

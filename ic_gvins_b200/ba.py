@@ -116,27 +116,16 @@ def merge_shard(prob: dict, shard: dict) -> None:
 
 
 def connect_shards(solver: "WindowSolver", rank: int, world: int, transport: str, dist) -> None:
-    """Join `solver` to the landmark-shard group of `world` processes (one per GPU).  `dist` is an initialised torch.distributed module
-    (any backend): it only carries the rendezvous blobs -- the ncclUniqueId for transport "nccl", the CUDA IPC handles of the exchange
-    buffers for transport "p2p" (peer-memory stores over NVLink, no NCCL on the data path)."""
-    if transport == "nccl":
-        ids = [nccl_unique_id() if rank == 0 else None]
-        dist.broadcast_object_list(ids, src=0)
-        solver.set_shard(rank, world, ids[0])
-    elif transport == "p2p":
-        mine = solver.shard_export(rank, world)
-        blobs = [None] * world
-        dist.all_gather_object(blobs, mine)
-        solver.shard_connect(blobs)
-        dist.barrier()
-    else:
+    """Join `solver` to the landmark-shard group of `world` processes (one per GPU).  The only transport is "p2p": peer-memory stores over
+    NVLink.  `dist` is an initialised torch.distributed module (any backend): it only carries the rendezvous blobs, the CUDA IPC handles of
+    the exchange buffers."""
+    if transport != "p2p":
         raise ValueError(transport)
-
-
-def nccl_unique_id() -> bytes:
-    buf = (C.c_uint8 * 128)()
-    check(lib().icg_nccl_unique_id(buf), "icg_nccl_unique_id")
-    return bytes(buf)
+    mine = solver.shard_export(rank, world)
+    blobs = [None] * world
+    dist.all_gather_object(blobs, mine)
+    solver.shard_connect(blobs)
+    dist.barrier()
 
 
 def imu_preintegrate(state16, iewn, gravity, noise5, imu):
@@ -170,11 +159,6 @@ class WindowSolver:
             self.close()
         except Exception:
             pass
-
-    def set_shard(self, rank: int, world: int, unique_id: bytes | None = None):
-        """Make this handle solve landmark shard `rank` of `world` (one process per GPU; NCCL all-reduce per LM attempt)."""
-        buf = (C.c_uint8 * 128)(*unique_id) if unique_id else None
-        check(lib().icg_ba_set_shard(self._h, rank, world, buf), "icg_ba_set_shard")
 
     def shard_export(self, rank: int, world: int) -> bytes:
         """Allocate this rank's peer-memory exchange buffer for a group of `world` ranks; returns the blob the other ranks need."""

@@ -16,7 +16,7 @@ LIB = os.path.join(HERE, "libicgvins_b200.so")
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 COMMON = ["-O3", "-lineinfo", "-std=c++17", "-Xcompiler", "-fPIC", "-Xcompiler", "-Wall", "-Xcompiler", "-Wno-unused-function"]
 # per-file extra flags: the image-path kernels must reproduce the reference library's float sequence (no FMA contraction)
-LINK_LIBS: list[str] = ["-ldl", "-lpthread"]  # cudart is linked statically (nvcc default); NCCL is dlopen-ed by ba.cu (headers only at build time)
+LINK_LIBS: list[str] = ["-ldl", "-lpthread"]  # cudart is linked statically (nvcc default) and needs both
 SOURCES = {
     "common.cu": [],
     "klt.cu": ["-fmad=false"],

@@ -21,10 +21,8 @@
 //                (panel updates on DMMA), triangular solves, landmark back-substitution, model cost change, candidate x (+) delta
 //   cost       : candidate cost (all factors, residuals only);   accept : Ceres step acceptance + radius update
 //   ba_marg.cuh: sliding-window marginalization (MarginalizationInfo) on the same device-resident linearisation
-#include <dlfcn.h>
 #include <unistd.h>
 #include <math.h>
-#include <nccl.h>
 #include <stdlib.h>
 #include <string.h>
 
@@ -104,10 +102,8 @@ struct BaDev {  // device pointers (flat, capacity-strided by window)
     int *marg_type, *marg_node;
     double *marg_x0, *marg_H0, *marg_b0, *marg_c0;
     double *cost_part;  // [NW][ncost_blocks]
-    double *red;        // [NW][2*NCA*NCA + 8]: vision Gram | Schur term | scalars -- the operand of the landmark-shard all-reduce
-    double *redmax;     // [NW] max |g_l| over the local landmarks (max-reduced)
-    double *red2;       // [NW][4]: model cost change, step norm^2, non-finite count, candidate cost (sum-reduced)
-    int rank, world;    // landmark shard of this process (camera-only terms are counted on rank 0 only)
+    double *red2;       // [NW][4]: model cost change, step norm^2, non-finite count, candidate cost
+    int rank, world;    // landmark shard of this process (split pipeline; 0 / 1 otherwise)
     double *step_c, *step_l;
     double *Sglobal;    // fallback Cholesky workspace when the packed system does not fit shared memory
     unsigned long long *clk;  // ICG_BA_PROFILE: SM-clock totals of ba_solve's phases for window 0 (nullptr otherwise)
@@ -367,24 +363,6 @@ __device__ __forceinline__ double gram2_entry(const BaCaps &C, const BaDev &D, i
     }
     return sum;
 }
-// stage 2 as its own kernel: landmark-sharded solves only (the vision Gram matrix must exist before the all-reduce)
-__global__ void __launch_bounds__(256) ba_pair_gram2(BaCaps C, BaDev D) {
-    __shared__ short s_slot[32 * 32];
-    const int w = blockIdx.y;
-    const LmState &st = D.st[w];
-    if (st.done || !st.need_lin) return;
-    const int K = D.dims[w].K, NCV = 6 * K + 7, nn = NCV + 1;
-    if ((int) blockIdx.x * 256 >= nn * nn) return;
-    gram2_slots(C, D, w, K, s_slot);
-    const int t = blockIdx.x * 256 + threadIdx.x;
-    if (t >= nn * nn) return;
-    const int A = t / nn, B = t - A * nn;
-    if (B < A) return;
-    const double sum = gram2_entry(C, D, w, K, s_slot, A, B);
-    double *Cout = D.CJ + (size_t) w * C.NCA * C.NCA;
-    Cout[(size_t) A * C.NCA + B] = sum;
-    Cout[(size_t) B * C.NCA + A] = sum;
-}
 
 // ------------------------------------------------------------------------------------------------ Schur term
 // Schur SYRK on the FP64 tensor cores: CW[split] = sum over the split's landmarks of phi_l w_l w_l^T (stored symmetric), with
@@ -392,7 +370,7 @@ __global__ void __launch_bounds__(256) ba_pair_gram2(BaCaps C, BaDev D) {
 // ba_pair_gram1 the A and B fragments of X^T X share one layout: lane reads A_W[l0 + lane%4][8 t + lane/4].  The CTA stages its
 // landmark rows (and phi) in shared memory once per pass -- leading dimension = 8 mod 16 doubles, so a fragment read is the minimal
 // two wavefronts -- and every warp accumulates two 16x16 super-tiles (2x2 DMMA tiles each) of the upper triangle per pass.
-// The BA_SPLIT_W landmark splits are separate CTAs whose partials ba_pack1 sums in fixed order (deterministic).
+// The BA_SPLIT_W landmark splits are separate CTAs whose partials ba_hsum / ba_export sum in fixed order (deterministic).
 constexpr int SCHUR_RCH = 80;  // landmark rows staged per chunk (multiple of 4)
 __device__ __forceinline__ void schur_body(const BaCaps &C, const BaDev &D, int w, int split, int ld, double *sA /* [SCHUR_RCH][ld] rows, then phi[SCHUR_RCH] */) {
     const LmState &st = D.st[w];
@@ -780,69 +758,9 @@ __global__ void __launch_bounds__(CAM_THREADS) ba_lin_cam(BaCaps C, BaDev D) {
     if (threadIdx.x == 0) st.cost_cam = c;
 }
 
-__device__ __forceinline__ double block_sum(double v, double *s_red);
-__device__ __forceinline__ double block_max(double v, double *s_red);
-
-// ------------------------------------------------------------------------------------------------ reduction operands
-// Everything a landmark shard contributes to the window's reduced camera system goes into ONE contiguous buffer per window, so that
-// a sharded solve needs a single all-reduce (sum) per attempt: [H_vis g_vis | Schur term | vision cost, sum rho^2].
-constexpr int PACK1_SPLIT = 4;  // CTAs per window
-__global__ void __launch_bounds__(256) ba_pack1(BaCaps C, BaDev D) {
-    __shared__ double s_red[40];
-    const int w = blockIdx.x, tid = threadIdx.x, part = blockIdx.y;
-    const LmState &st = D.st[w];
-    if (st.done) return;
-    const WinDims dm = D.dims[w];
-    const int NN = C.NCA * C.NCA;
-    double *R = D.red + (size_t) w * (2 * NN + 8);
-    const double *CJ = D.CJ + (size_t) w * BA_SPLIT_J * NN, *CW = D.CW + (size_t) w * BA_SPLIT_W * NN;
-    const int e0 = (int) ((long long) NN * part / PACK1_SPLIT), e1 = (int) ((long long) NN * (part + 1) / PACK1_SPLIT);
-    for (int e = e0 + tid; e < e1; e += 256) {
-        const double cj = CJ[e];
-        double p[BA_SPLIT_W];
-#pragma unroll
-        for (int k = 0; k < BA_SPLIT_W; k++) p[k] = CW[(size_t) k * NN + e];
-        double s = 0;
-#pragma unroll
-        for (int k = 0; k < BA_SPLIT_W; k++) s += p[k];
-        R[e] = cj;
-        R[NN + e] = s;
-    }
-    if (part != 0) return;
-    double c = 0, q = 0, gm = 0;
-    for (int f = tid; f < dm.F; f += 256) c += D.costf[(size_t) w * C.F + f];
-    for (int l = tid; l < dm.L; l += 256) {
-        const double r = D.rho[(size_t) w * C.L + l];
-        q += r * r;
-        gm = fmax(gm, fabs(D.gl[(size_t) w * C.L + l]));
-    }
-    c = block_sum(c, s_red);
-    q = block_sum(q, s_red);
-    gm = block_max(gm, s_red);
-    if (tid == 0) {
-        R[2 * NN] = c, R[2 * NN + 1] = q;
-        for (int k = 2; k < 8; k++) R[2 * NN + k] = 0;
-        D.redmax[w] = gm;
-    }
-}
-
-__global__ void ba_pack2(BaCaps C, BaDev D, int n, int nblk_vis) {
-    const int w = blockIdx.x * blockDim.x + threadIdx.x;
-    if (w >= n) return;
-    const LmState &st = D.st[w];
-    if (st.done || !st.step_valid) return;
-    const WinDims dm = D.dims[w];
-    const double *part = D.cost_part + (size_t) w * (nblk_vis + 1);
-    double cand = 0;
-    const int nb = (dm.F + 255) / 256;
-    for (int b = 0; b < nb; b++) cand += part[b];
-    if (D.rank == 0) cand += part[nblk_vis];  // camera-only factors are replicated on every shard: count them once
-    D.red2[(size_t) w * 4 + 3] = cand;
-}
-
 // ------------------------------------------------------------------------------------------------ reduced camera matrix
 // Hs = H_c + H_vis - Schur term, lower triangle, one thread per entry (wide and coalesced; ba_solve then reads ONE operand per entry
-// instead of gathering 2 + BA_SPLIT_W).  Landmark-sharded solve: the vision / Schur operands are the all-reduced buffer.
+// instead of gathering 2 + BA_SPLIT_W).  The gather of the per-pair Gram matrices happens here too, one kernel less on the path.
 __global__ void __launch_bounds__(256) ba_hsum(BaCaps C, BaDev D) {
     __shared__ short s_slot[32 * 32];
     const int w = blockIdx.y;
@@ -850,27 +768,19 @@ __global__ void __launch_bounds__(256) ba_hsum(BaCaps C, BaDev D) {
     const int K = D.dims[w].K, NCV = 6 * K + 7, nn = NCV + 1;
     const int NN = C.NCA * C.NCA;
     if ((int) blockIdx.x * 256 >= nn * nn) return;
-    const bool sharded = D.world > 1;
-    if (!sharded) gram2_slots(C, D, w, K, s_slot);
+    gram2_slots(C, D, w, K, s_slot);
     const int t = blockIdx.x * 256 + threadIdx.x;
     if (t >= nn * nn) return;
     const int A = t / nn, B = t - A * nn;  // A <= B: entry (row B, column A) of the lower triangle
     if (B < A) return;
-    double cj, cw;
-    if (sharded) {
-        const double *RED = D.red + (size_t) w * (2 * NN + 8);
-        cj = RED[(size_t) B * C.NCA + A], cw = RED[NN + (size_t) B * C.NCA + A];
-    } else {
-        // single GPU: the gather of the per-pair Gram matrices (ba_pair_gram2's job) happens here, one kernel less on the path
-        cj = gram2_entry(C, D, w, K, s_slot, A, B);
-        double *Cout = D.CJ + (size_t) w * NN;
-        Cout[(size_t) A * C.NCA + B] = cj;
-        Cout[(size_t) B * C.NCA + A] = cj;
-        const double *CWp = D.CW + (size_t) w * BA_SPLIT_W * NN;
-        cw = 0;
+    const double cj = gram2_entry(C, D, w, K, s_slot, A, B);
+    double *Cout = D.CJ + (size_t) w * NN;
+    Cout[(size_t) A * C.NCA + B] = cj;
+    Cout[(size_t) B * C.NCA + A] = cj;
+    const double *CWp = D.CW + (size_t) w * BA_SPLIT_W * NN;
+    double cw = 0;
 #pragma unroll
-        for (int k = 0; k < BA_SPLIT_W; k++) cw += CWp[(size_t) k * NN + (size_t) B * C.NCA + A];
-    }
+    for (int k = 0; k < BA_SPLIT_W; k++) cw += CWp[(size_t) k * NN + (size_t) B * C.NCA + A];
     if (B < NCV) D.Hs[(size_t) w * C.NS * C.NS + (size_t) B * C.NS + A] = D.Hc[(size_t) w * C.NS * C.NS + (size_t) B * C.NS + A] + (cj - cw);
 }
 
@@ -946,21 +856,16 @@ __global__ void __launch_bounds__(SOLVE_THREADS, 2) ba_solve(BaCaps C, BaDev D) 
     // pointer that could also be global made every access a generic LD / ST (longer latency, long-scoreboard tracked)
     double *S = s_diag + C.NS;
     const double *Hc = D.Hc + (size_t) w * C.NS * C.NS, *gcam = D.gc + (size_t) w * C.NS, *Hs = D.Hs + (size_t) w * C.NS * C.NS;
-    // Reduction operands.  Landmark-sharded solve: the packed, all-reduced buffer (identical on every shard, written by ba_pack1).
-    // Single GPU: read the producers' outputs directly (vision Gram matrix; the BA_SPLIT_W Schur partials summed in fixed order).
-    const bool sharded = D.world > 1;
+    // Reduction operands: the producers' outputs, read directly (vision Gram matrix; the BA_SPLIT_W Schur partials summed in fixed order).
     const int NN = C.NCA * C.NCA;
-    const double *RED = D.red + (size_t) w * (2 * NN + 8);
-    const double *CJ = sharded ? RED : D.CJ + (size_t) w * BA_SPLIT_J * NN;
-    const double *CWp = sharded ? RED + NN : D.CW + (size_t) w * BA_SPLIT_W * NN;
+    const double *CJ = D.CJ + (size_t) w * BA_SPLIT_J * NN;
+    const double *CWp = D.CW + (size_t) w * BA_SPLIT_W * NN;
     auto cw_get = [&](int a, int b) {  // symmetric storage: any (a, b)
-        if (sharded) return CWp[(size_t) a * C.NCA + b];
         double s2 = 0;
 #pragma unroll
         for (int k = 0; k < BA_SPLIT_W; k++) s2 += CWp[(size_t) k * NN + (size_t) a * C.NCA + b];
         return s2;
     };
-    const double camw = D.rank == 0 ? 1.0 : 0.0;       // camera-side partial sums are counted on shard 0 only
     if (tid == 0 && st.need_lin) st.need_lin = 0;      // the linearisation kernels of this iteration have run (stream order)
     double *scale_c = D.scale_c + (size_t) w * C.NS;
     const double *hl = D.hl + (size_t) w * C.L, *gl = D.gl + (size_t) w * C.L, *scale_l = D.scale_l + (size_t) w * C.L;
@@ -979,17 +884,11 @@ __global__ void __launch_bounds__(SOLVE_THREADS, 2) ba_solve(BaCaps C, BaDev D) 
     for (int a = tid; a < N; a += SOLVE_THREADS) s_scale[a] = scale_c[a];
     double gmax_now = st.gmax;
     if (f_fresh) {
-        double c, gml;
-        if (sharded) {
-            c = RED[2 * NN];  // vision cost, summed over the landmark shards
-            gml = D.redmax[w];
-        } else {
-            double cs = 0, gq = 0;
-            for (int f = tid; f < dm.F; f += SOLVE_THREADS) cs += D.costf[(size_t) w * C.F + f];
-            for (int l = tid; l < L; l += SOLVE_THREADS) gq = fmax(gq, fabs(gl[l]));
-            c = block_sum(cs, s_red);
-            gml = block_max(gq, s_red);
-        }
+        double cs = 0, gq = 0;
+        for (int f = tid; f < dm.F; f += SOLVE_THREADS) cs += D.costf[(size_t) w * C.F + f];
+        for (int l = tid; l < L; l += SOLVE_THREADS) gq = fmax(gq, fabs(gl[l]));
+        const double c = block_sum(cs, s_red);
+        const double gml = block_max(gq, s_red);
         double gm = 0;
         for (int a = tid; a < N; a += SOLVE_THREADS) gm = fmax(gm, fabs(s_g[a]));
         gm = fmax(block_max(gm, s_red), gml);
@@ -1294,7 +1193,7 @@ __global__ void __launch_bounds__(SOLVE_THREADS, 2) ba_solve(BaCaps C, BaDev D) 
     bool finite = true;
     double *R2 = D.red2 + (size_t) w * 4;
     if (!valid) {
-        // Cholesky breakdown (identical on every shard): the step is invalid; ba_accept applies HandleInvalidStep
+        // Cholesky breakdown: the step is invalid; ba_accept applies HandleInvalidStep
         if (tid == 0) {
             st.chol_ok = 0, st.step_valid = 0;
             R2[0] = 0, R2[1] = 0, R2[2] = 1, R2[3] = 0;
@@ -1304,7 +1203,7 @@ __global__ void __launch_bounds__(SOLVE_THREADS, 2) ba_solve(BaCaps C, BaDev D) 
     for (int a = tid; a < N; a += SOLVE_THREADS) {
         double sp = s_rhs[a];
         finite = finite && isfinite(sp);
-        part += camw * (-0.5 * sp * (s_scale[a] * s_g[a]) + 0.5 * s_d2[a] * sp * sp);
+        part += -0.5 * sp * (s_scale[a] * s_g[a]) + 0.5 * s_d2[a] * sp * sp;
     }
     // landmark back-substitution: one warp per landmark, the coupling row is read coalesced (two landmarks in flight per warp)
     double *s_sx = s_diag;  // s_diag is dead after the back-substitution: scaled camera step s_c * step'_c
@@ -1368,7 +1267,7 @@ __global__ void __launch_bounds__(SOLVE_THREADS, 2) ba_solve(BaCaps C, BaDev D) 
     SOLVE_CLK(4)  // landmark back-substitution
     const double mcc = block_sum(part, s_red);
     const double nfin = block_sum(finite ? 0.0 : 1.0, s_red);
-    // ---- candidate point x (+) delta, delta = step' * scale; |x - x_cand|^2 over active blocks (camera part counted on shard 0)
+    // ---- candidate point x (+) delta, delta = step' * scale; |x - x_cand|^2 over active blocks
     const double *pose = D.pose + (size_t) w * C.K * 7, *mix = D.mix + (size_t) w * C.K * 9, *ext = D.ext + (size_t) w * 8, *rho = D.rho + (size_t) w * C.L;
     double *pose_c = D.pose_c + (size_t) w * C.K * 7, *mix_c = D.mix_c + (size_t) w * C.K * 9, *ext_c = D.ext_c + (size_t) w * 8, *rho_c = D.rho_c + (size_t) w * C.L;
     double sn = 0;
@@ -1383,14 +1282,14 @@ __global__ void __launch_bounds__(SOLVE_THREADS, 2) ba_solve(BaCaps C, BaDev D) 
             double d[6];
             for (int e = 0; e < 6; e++) d[e] = s_rhs[c0 + e] * s_scale[c0 + e];
             pose_plus(x, d, xc);
-            for (int e = 0; e < 7; e++) sn += camw * (x[e] - xc[e]) * (x[e] - xc[e]);
+            for (int e = 0; e < 7; e++) sn += (x[e] - xc[e]) * (x[e] - xc[e]);
         }
     }
     for (int e = tid; e < K * 9; e += SOLVE_THREADS) {
         int k = e / 9, q = e - 9 * k, c = col_mix(K, k) + q;
         double v = mix[e] + s_rhs[c] * s_scale[c];
         mix_c[e] = v;
-        sn += camw * (mix[e] - v) * (mix[e] - v);
+        sn += (mix[e] - v) * (mix[e] - v);
     }
     if (tid == 0) {
         if (dm.td_const) {
@@ -1398,7 +1297,7 @@ __global__ void __launch_bounds__(SOLVE_THREADS, 2) ba_solve(BaCaps C, BaDev D) 
         } else {
             double v = ext[7] + s_rhs[col_td(K)] * s_scale[col_td(K)];
             ext_c[7] = v;
-            sn += camw * (ext[7] - v) * (ext[7] - v);
+            sn += (ext[7] - v) * (ext[7] - v);
         }
     }
     for (int l = tid; l < L; l += SOLVE_THREADS) {
@@ -1469,7 +1368,7 @@ __global__ void __launch_bounds__(128) ba_accept(BaCaps C, BaDev D, int nblk_vis
     const WinDims dm = D.dims[w];
     const int chol_ok = st.chol_ok;
     const double *R2 = D.red2 + (size_t) w * 4;
-    // |x|^2 of the camera-side blocks (replicated on every shard); the landmark part comes from the reduced operand
+    // |x|^2 of the camera-side blocks and of the inverse depths
     {
         const double *pose = D.pose + (size_t) w * C.K * 7, *mix = D.mix + (size_t) w * C.K * 9, *ext = D.ext + (size_t) w * 8;
         double s = 0;
@@ -1478,13 +1377,9 @@ __global__ void __launch_bounds__(128) ba_accept(BaCaps C, BaDev D, int nblk_vis
         if (tid < 7 && !dm.ext_const) s += ext[tid] * ext[tid];
         if (tid == 7 && !dm.td_const) s += ext[7] * ext[7];
         s = block_sum(s, s_red);
-        double q = 0;  // |rho|^2: from the reduced operand when the landmarks are sharded
-        if (D.world == 1) {
-            for (int l = tid; l < dm.L; l += 128) q += D.rho[(size_t) w * C.L + l] * D.rho[(size_t) w * C.L + l];
-            q = block_sum(q, s_red);
-        } else {
-            q = D.red[(size_t) w * (2 * C.NCA * C.NCA + 8) + 2 * C.NCA * C.NCA + 1];
-        }
+        double q = 0;
+        for (int l = tid; l < dm.L; l += 128) q += D.rho[(size_t) w * C.L + l] * D.rho[(size_t) w * C.L + l];
+        q = block_sum(q, s_red);
         if (tid == 0) s_camsq = s, s_rhosq = q;
     }
     __syncthreads();
@@ -1492,7 +1387,7 @@ __global__ void __launch_bounds__(128) ba_accept(BaCaps C, BaDev D, int nblk_vis
         s_accept = 0;
         const double mcc = R2[0], sn = R2[1], nfin = R2[2];
         double cand = R2[3];
-        if (D.world == 1 && st.step_valid) {  // single GPU: sum the candidate-cost partials here (ba_pack2 does it before the all-reduce otherwise)
+        if (st.step_valid) {  // sum the candidate-cost partials (vision blocks, then the camera-only factors)
             const double *part = D.cost_part + (size_t) w * (nblk_vis + 1);
             cand = 0;
             const int nb = (dm.F + 255) / 256;
@@ -1776,7 +1671,7 @@ struct icg_ba {
     bool own_stream = false;
     int nblk_vis = 0;
     int cur_windows = 0;
-    int cam_threads = 160;  // CTA size of the camera-only factor kernels (<= CAM_THREADS; ICG_BA_CAM_THREADS): 160 x 168 registers leave room for two
+    int cam_threads = 160;  // CTA size of the camera-only factor kernels (<= CAM_THREADS): 160 x 168 registers leave room for two
                             // ba_lin_vis CTAs on the SM (320 threads take 82 % of the register file: nothing else fits beside them)
     size_t smem_cam, smem_solve, smem_schur;
     int ld_schur;
@@ -1793,18 +1688,15 @@ struct icg_ba {
     HostDev<double> scratch;  // single-factor evaluation
     HostDev<LmState> st_save;   // pass-1 LM state of the two-pass protocol
     HostDev<int> cull_counters; // per window: reprojection factors removed, GNSS fixes re-weighted
-    void *comm = nullptr;       // ncclComm_t when this handle solves a landmark shard (transport "nccl")
     // split pipeline (ba_split.cuh): exchange buffer of this rank, peers' buffers opened through CUDA IPC, epoch counter of the flags
     double *xbuf = nullptr;
     size_t xbuf_doubles = 0;
-    int x_world = 0;
     void *ipc_opened[8] = {nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, nullptr};
     unsigned long long epoch = 0;
     size_t smem_solve_cam = 0, smem_step_lm = 0;
     bool solve_cam_stage_a = false;  // per-warp shared-memory strips for the DMMA A operand (ba_solve_cam)
     bool solve_cam_dsm = false;      // the packed system fits the cluster's shared memory: ba_solve_cam_dsm (max_K <= 22)
     size_t smem_solve_cam_dsm = 0;
-    int dsm_variant = 0;             // ba_solve_cam_dsm: DSM_V_* bits (ICG_BA_DSM_VARIANT)
     // in-situ stage timing (ICG_BA_PROFILE=1): events between the kernels of the LM sequence on the main stream, read back in
     // icg_ba_sync / icg_ba_download and printed by icg_ba_destroy (warm caches, real launch gaps -- unlike an ncu replay)
     bool prof = false;
@@ -1837,43 +1729,6 @@ static int dmalloc(icg_ba *h, double **p, size_t n) {
     h->dev_only.push_back(*p);
     return ICG_OK;
 }
-
-// ---- NCCL, loaded at run time (only landmark-sharded solves need it; the KLT / single-GPU paths never touch it)
-namespace {
-struct NcclApi {
-    void *lib = nullptr;
-    ncclResult_t (*GetUniqueId)(ncclUniqueId *) = nullptr;
-    ncclResult_t (*CommInitRank)(ncclComm_t *, int, ncclUniqueId, int) = nullptr;
-    ncclResult_t (*AllReduce)(const void *, void *, size_t, ncclDataType_t, ncclRedOp_t, ncclComm_t, cudaStream_t) = nullptr;
-    ncclResult_t (*CommDestroy)(ncclComm_t) = nullptr;
-    const char *(*GetErrorString)(ncclResult_t) = nullptr;
-};
-NcclApi &nccl_api() {
-    static NcclApi api;
-    if (!api.lib) {
-        api.lib = dlopen("libnccl.so.2", RTLD_NOW | RTLD_GLOBAL);
-        if (api.lib) {
-            api.GetUniqueId = (decltype(api.GetUniqueId)) dlsym(api.lib, "ncclGetUniqueId");
-            api.CommInitRank = (decltype(api.CommInitRank)) dlsym(api.lib, "ncclCommInitRank");
-            api.AllReduce = (decltype(api.AllReduce)) dlsym(api.lib, "ncclAllReduce");
-            api.CommDestroy = (decltype(api.CommDestroy)) dlsym(api.lib, "ncclCommDestroy");
-            api.GetErrorString = (decltype(api.GetErrorString)) dlsym(api.lib, "ncclGetErrorString");
-        }
-    }
-    return api;
-}
-}  // namespace
-
-static int nccl_allreduce(icg_ba *h, double *buf, size_t count, int op_max) {
-    NcclApi &a = nccl_api();
-    ncclResult_t r = a.AllReduce(buf, buf, count, ncclDouble, op_max ? ncclMax : ncclSum, (ncclComm_t) h->comm, h->stream);
-    if (r != ncclSuccess) {
-        set_error("ncclAllReduce failed: %s", a.GetErrorString ? a.GetErrorString(r) : "?");
-        return ICG_ENCCL;
-    }
-    return ICG_OK;
-}
-
 
 extern "C" {
 static int split_setup(icg_ba *h, int rank, int world);
@@ -1944,7 +1799,6 @@ static int ba_create_body(icg_ba *h, int max_windows, int max_K, int max_L, int 
     ICG_CUDA(cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming));
     ICG_CUDA(cudaEventCreateWithFlags(&h->ev_join, cudaEventDisableTiming));
     h->prof = getenv("ICG_BA_PROFILE") != nullptr;
-    if (getenv("ICG_BA_CAM_THREADS")) h->cam_threads = std::min(CAM_THREADS, std::max(128, atoi(getenv("ICG_BA_CAM_THREADS")) & ~31));
     if (h->prof) {
         double *ck = nullptr;
         if (dmalloc(h, &ck, 48) != ICG_OK) return ICG_ENOMEM;
@@ -1989,7 +1843,7 @@ static int ba_create_body(icg_ba *h, int max_windows, int max_K, int max_L, int 
     DM(pose_0, NW * C.K * 7) DM(mix_0, NW * C.K * 9) DM(ext_0, NW * 8) DM(rho_0, NW * C.L)
     DM(AW, NW * C.NCA * C.LP) DM(Mp, NW * (size_t) C.K * (C.K - 1) * 210) DM(CJ, NW * BA_SPLIT_J * C.NCA * C.NCA) DM(CW, NW * BA_SPLIT_W * C.NCA * C.NCA)
     DM(jcomp, NW * C.F * 40) DM(costf, NW * C.F) DM(hl, NW * C.L) DM(gl, NW * C.L) DM(scale_l, NW * C.L) DM(scale_c, NW * C.NS)
-    DM(Hc, NW * C.NS * C.NS) DM(gc, NW * C.NS) DM(Hs, NW * C.NS * C.NS) DM(cost_part, NW * (h->nblk_vis + 1)) DM(red, NW * (2 * (size_t) C.NCA * C.NCA + 8)) DM(redmax, NW) DM(red2, NW * 4) DM(step_c, NW * C.NS) DM(step_l, NW * C.L)
+    DM(Hc, NW * C.NS * C.NS) DM(gc, NW * C.NS) DM(Hs, NW * C.NS * C.NS) DM(cost_part, NW * (h->nblk_vis + 1)) DM(red2, NW * 4) DM(step_c, NW * C.NS) DM(step_l, NW * C.L)
 #undef DM
     if (rc == ICG_OK) rc = dmalloc(h, &D.gnss_std_0, NW * C.G * 3);
     if (rc == ICG_OK) {
@@ -2036,7 +1890,6 @@ void icg_ba_destroy(icg_ba *h) {
     h->pose_prior_sinfo.release(), h->mix_prior.release(), h->mix_prior_std.release(), h->marg_x0.release(), h->marg_H0.release(), h->marg_b0.release();
     h->marg_c0.release(), h->lm_off.release(), h->lm_fidx.release(), h->gnss_node.release();
     h->f_slot.release(), h->f_meta_s.release(), h->vb_lm0.release(), h->f_const_s.release(), h->marg_type.release(), h->marg_node.release(), h->f_active.release(), h->scratch.release(), h->st_save.release(), h->cull_counters.release(), h->pair_off.release(), h->pair_ro.release(), h->pair_fidx.release(), h->npairs.release();
-    if (h->comm) nccl_api().CommDestroy((ncclComm_t) h->comm);
     split_release(h);
     if (h->marg_ready) h->marg_map.release(), h->marg_oJ0.release(), h->marg_oe0.release(), h->marg_oHp.release(), h->marg_obp.release();
     h->cull_buf.release();
@@ -2263,8 +2116,8 @@ int icg_ba_upload(icg_ba *h, int n, const icg_ba_problem *P) {
 }
 
 // ---- in-situ stage timing
-static const char *PROF_NAMES[16] = {"(gap/other)", "lin_vis", "lin_lm", "pair_gram1", "pair_gram2", "schur_dmma", "join lin_cam + lin_done",
-                                     "pack1 / export + signal", "solve", "cost (+cost_cam)", "pack2 / exchange", "accept", "hsum / reduce", "join gram chain", "step_lm", ""};
+static const char *PROF_NAMES[16] = {"(gap/other)", "lin_vis", "lin_lm", "pair_gram1", "", "schur_dmma", "join lin_cam + lin_done",
+                                     "export + signal", "solve", "cost (+cost_cam)", "exchange", "accept", "hsum / reduce", "join gram chain", "step_lm", ""};
 static void prof_mark(icg_ba *h, int tag) {
     if (!h->prof) return;
     if (h->prof_used == h->prof_ev.size()) {
@@ -2338,51 +2191,29 @@ static int enqueue_lm(icg_ba *h, int max_num_iterations) {
     const dim3 g_vis(C.NVB - 2, n), g_cost(h->nblk_vis, n);
     // iteration 0 linearisation + (max_iter) x [schur syrk, solve, cost, accept, re-linearise]; one extra solve call
     // performs the final termination bookkeeping.
-    // where the camera-only factors are forked: 0 = beside ba_lin_vis (round 1), 1 = behind it, beside the Schur / Gram kernels (ba_lin_vis holds
-    // 128 registers x 4 CTAs: a 320-thread camera CTA on the same SM costs it a resident CTA).  Chosen by measurement (profiles/r2_ba_stages.md).
-    static const int cam_fork = getenv("ICG_BA_CAM_FORK") ? atoi(getenv("ICG_BA_CAM_FORK")) : 0;
     for (int it = 0; it <= max_num_iterations; it++) {
-        // fork: IMU / GNSS / prior factors (one latency-bound CTA per window) run beside the vision chain
-        if (cam_fork == 0) {
-            ICG_CUDA(cudaEventRecord(h->ev_fork, s));
-            ICG_CUDA(cudaStreamWaitEvent(h->stream_cam, h->ev_fork, 0));
-            ba_lin_cam<<<n, h->cam_threads, h->smem_cam, h->stream_cam>>>(C, D);
-            ICG_CUDA(cudaEventRecord(h->ev_join, h->stream_cam));
-        }
+        // fork: IMU / GNSS / prior factors (one latency-bound CTA per window) run beside the vision chain, from ba_lin_vis on (measured
+        // against forking them beside the Schur / Gram kernels instead: profiles/r2_ba_stages.md)
+        ICG_CUDA(cudaEventRecord(h->ev_fork, s));
+        ICG_CUDA(cudaStreamWaitEvent(h->stream_cam, h->ev_fork, 0));
+        ba_lin_cam<<<n, h->cam_threads, h->smem_cam, h->stream_cam>>>(C, D);
+        ICG_CUDA(cudaEventRecord(h->ev_join, h->stream_cam));
         prof_mark(h, 0);
         ba_lin_vis<<<g_vis, 128, LV_SMEM, s>>>(C, D);
         prof_mark(h, 1);
-        if (cam_fork != 0) {
-            ICG_CUDA(cudaEventRecord(h->ev_fork, s));
-            ICG_CUDA(cudaStreamWaitEvent(h->stream_cam, h->ev_fork, 0));
-            ba_lin_cam<<<n, h->cam_threads, h->smem_cam, h->stream_cam>>>(C, D);
-            ICG_CUDA(cudaEventRecord(h->ev_join, h->stream_cam));
-        }
         // (measured: one fused launch or two streams are both slower -- the Schur CTAs' shared memory throttles the latency-bound
         //  Gram warps when they share SMs)
         ba_schur_dmma<<<dim3(BA_SPLIT_W, n), 256, h->smem_schur, s>>>(C, D, h->ld_schur);
         prof_mark(h, 5);
         ba_pair_gram1<<<dim3((C.K * (C.K - 1) + 7) / 8, n), 256, 0, s>>>(C, D);
         prof_mark(h, 3);
-        if (h->comm) {
-            ba_pair_gram2<<<dim3(((C.NCV + 1) * (C.NCV + 1) + 255) / 256, n), 256, 0, s>>>(C, D);
-            prof_mark(h, 4);
-        }
         ICG_CUDA(cudaStreamWaitEvent(s, h->ev_join, 0));
         prof_mark(h, 6);
-        if (h->comm) {  // landmark-sharded window: one sum all-reduce of [H_vis g | Schur | cost, |rho|^2] + one max all-reduce
-            ba_pack1<<<dim3(n, PACK1_SPLIT), 256, 0, s>>>(C, D);
-            prof_mark(h, 7);
-            int rc = nccl_allreduce(h, D.red, (size_t) n * (2 * (size_t) C.NCA * C.NCA + 8), 0);
-            if (rc != ICG_OK) return rc;
-            rc = nccl_allreduce(h, D.redmax, (size_t) n, 1);
-            if (rc != ICG_OK) return rc;
-        }
         ba_hsum<<<dim3(((C.NCV + 1) * (C.NCV + 1) + 255) / 256, n), 256, 0, s>>>(C, D);
         prof_mark(h, 12);
         ba_solve<<<n, SOLVE_THREADS, h->smem_solve, s>>>(C, D);
         prof_mark(h, 8);
-        count_launch(h->comm ? 8 : 6);
+        count_launch(6);
         if (it == max_num_iterations) break;
         ICG_CUDA(cudaEventRecord(h->ev_fork, s));
         ICG_CUDA(cudaStreamWaitEvent(h->stream_cam, h->ev_fork, 0));
@@ -2391,15 +2222,9 @@ static int enqueue_lm(icg_ba *h, int max_num_iterations) {
         ba_cost<<<g_cost, 256, 0, s>>>(C, D, h->nblk_vis);
         ICG_CUDA(cudaStreamWaitEvent(s, h->ev_join, 0));
         prof_mark(h, 9);
-        if (h->comm) {
-            ba_pack2<<<(n + 127) / 128, 128, 0, s>>>(C, D, n, h->nblk_vis);
-            prof_mark(h, 10);
-            int rc = nccl_allreduce(h, D.red2, (size_t) n * 4, 0);
-            if (rc != ICG_OK) return rc;
-        }
         ba_accept<<<n, 128, 0, s>>>(C, D, h->nblk_vis);
         prof_mark(h, 11);
-        count_launch(h->comm ? 4 : 3);
+        count_launch(3);
     }
     ICG_CHECK_LAUNCH();
     return ICG_OK;
@@ -2460,11 +2285,10 @@ static int split_setup(icg_ba *h, int rank, int world) {
     S.peer[rank] = h->xbuf;
     S.split = 1;
     h->D.rank = rank, h->D.world = world;
-    h->x_world = world;
     // four or more landmark shards: the owner's camera-only kernels are on the attempt's critical path (the vision kernels shrink with the
     // shard -- 410 us at one rank, ~100 at four --, the per-window IMU chain of ~118 us does not): all 10 warps, two rounds of IMU factors at
     // K = 20 instead of four
-    if (!getenv("ICG_BA_CAM_THREADS")) h->cam_threads = world >= 4 ? CAM_THREADS : 160;
+    h->cam_threads = world >= 4 ? CAM_THREADS : 160;
     h->epoch = 0;
     {   // ba_solve_cam: vectors + the larger of the back-substitution staging and [B rows | 8 x 8 hand-over | one A strip per warp]; the A strips are
         // dropped when they do not fit (max_K > 20)
@@ -2475,9 +2299,8 @@ static int split_setup(icg_ba *h, int rank, int world) {
     }
     h->smem_step_lm = sizeof(double) * (40 + (size_t) C.NS);
     h->smem_solve_cam_dsm = sizeof(double) * dsm_smem_doubles(C);
-    h->solve_cam_dsm = h->smem_solve_cam_dsm <= 227 * 1024 && C.N <= 32 * 11 && !getenv("ICG_BA_SOLVE_CAM_L2");  // (the assembly stages <= 11 chunks of 32 columns per row)
+    h->solve_cam_dsm = h->smem_solve_cam_dsm <= 227 * 1024 && C.N <= 32 * 11;  // (the assembly stages <= 11 chunks of 32 columns per row)
     if (h->solve_cam_dsm) ICG_CUDA(raise_dynamic_smem((const void *) ba_solve_cam_dsm, h->smem_solve_cam_dsm));
-    h->dsm_variant = getenv("ICG_BA_DSM_VARIANT") ? atoi(getenv("ICG_BA_DSM_VARIANT")) : DSM_V_MBAR_BSUB;
     ICG_CUDA(raise_dynamic_smem((const void *) ba_solve_cam, (size_t) (h->smem_solve_cam)));
     ICG_CUDA(cudaFuncSetAttribute(ba_solve_cam, cudaFuncAttributeNonPortableClusterSizeAllowed, 0));
     ICG_CUDA(raise_dynamic_smem((const void *) ba_step_lm, (size_t) (h->smem_step_lm)));
@@ -2493,7 +2316,7 @@ static int launch_solve_cam(icg_ba *h, int n, unsigned long long epoch) {
     at[0].id = cudaLaunchAttributeClusterDimension;
     at[0].val.clusterDim.x = SPLIT_CLUSTER, at[0].val.clusterDim.y = 1, at[0].val.clusterDim.z = 1;
     cfg.attrs = at, cfg.numAttrs = 1;
-    if (h->solve_cam_dsm) ICG_CUDA(cudaLaunchKernelEx(&cfg, ba_solve_cam_dsm, h->C, h->D, epoch, h->dsm_variant));
+    if (h->solve_cam_dsm) ICG_CUDA(cudaLaunchKernelEx(&cfg, ba_solve_cam_dsm, h->C, h->D, epoch));
     else ICG_CUDA(cudaLaunchKernelEx(&cfg, ba_solve_cam, h->C, h->D, epoch, (int) h->solve_cam_stage_a));
     return ICG_OK;
 }
@@ -2750,8 +2573,8 @@ static int marginalize_body(icg_ba *h, int n_windows, const icg_ba_problem *prob
         set_error("icg_ba_marginalize: bad arguments");
         return ICG_EINVAL;
     }
-    if (h->comm || h->D.world > 1) {
-        set_error("icg_ba_marginalize: not available on a landmark-sharded handle (icg_ba_set_shard(world = 1) first)");
+    if (h->D.world > 1) {
+        set_error("icg_ba_marginalize: not available on a landmark-sharded handle");
         return ICG_EUNSUPPORTED;
     }
     int rc = ICG_OK;
@@ -2948,8 +2771,8 @@ int icg_ba_outlier_culling_resident(icg_ba *h, int n_windows, const icg_ba_probl
         set_error("icg_ba_outlier_culling_resident: bad arguments");
         return ICG_EINVAL;
     }
-    if (h->comm || h->D.world > 1) {
-        set_error("icg_ba_outlier_culling_resident: not available on a landmark-sharded handle (icg_ba_set_shard(world = 1) first)");
+    if (h->D.world > 1) {
+        set_error("icg_ba_outlier_culling_resident: not available on a landmark-sharded handle");
         return ICG_EUNSUPPORTED;
     }
     if (h->cur_windows != n_windows) {
@@ -3060,60 +2883,6 @@ int icg_ba_outlier_culling_resident(icg_ba *h, int n_windows, const icg_ba_probl
     return ICG_OK;
 }
 
-int icg_nccl_unique_id(uint8_t *id128) {
-    NcclApi &a = nccl_api();
-    if (!a.lib || !a.GetUniqueId) {
-        set_error("icg_nccl_unique_id: libnccl.so.2 not loadable");
-        return ICG_ENCCL;
-    }
-    ncclUniqueId id;
-    ncclResult_t r = a.GetUniqueId(&id);
-    if (r != ncclSuccess) {
-        set_error("ncclGetUniqueId failed: %s", a.GetErrorString(r));
-        return ICG_ENCCL;
-    }
-    static_assert(sizeof(ncclUniqueId) == 128, "ncclUniqueId size");
-    memcpy(id128, &id, 128);
-    return ICG_OK;
-}
-
-int icg_ba_set_shard(icg_ba *h, int rank, int world, const uint8_t *id128) {
-    if (!h || rank < 0 || world < 1 || rank >= world) {
-        set_error("icg_ba_set_shard: bad arguments");
-        return ICG_EINVAL;
-    }
-    ICG_CUDA(cudaSetDevice(h->device));
-    NcclApi &a = nccl_api();
-    if (h->comm) {
-        a.CommDestroy((ncclComm_t) h->comm);
-        h->comm = nullptr;
-    }
-    if (h->D.S.split && h->x_world > 1) {  // leaving a peer-memory shard group
-        int rc = h->use_global_S ? split_setup(h, 0, 1) : (split_release(h), ICG_OK);
-        if (rc != ICG_OK) return rc;
-    }
-    if (world > 1 && h->use_global_S) {
-        set_error("icg_ba_set_shard: windows of this size (max_K = %d) are solved by the split pipeline; use icg_ba_shard_export / icg_ba_shard_connect (transport p2p)", h->C.K);
-        return ICG_EUNSUPPORTED;
-    }
-    h->D.rank = rank, h->D.world = world;
-    if (world == 1) return ICG_OK;
-    if (!id128 || !a.lib || !a.CommInitRank) {
-        set_error("icg_ba_set_shard: libnccl.so.2 not loadable or null id");
-        return ICG_ENCCL;
-    }
-    ncclUniqueId id;
-    memcpy(&id, id128, 128);
-    ncclComm_t comm;
-    ncclResult_t r = a.CommInitRank(&comm, world, id, rank);
-    if (r != ncclSuccess) {
-        set_error("ncclCommInitRank failed: %s", a.GetErrorString(r));
-        return ICG_ENCCL;
-    }
-    h->comm = comm;
-    return ICG_OK;
-}
-
 // ---- landmark shards over peer memory (transport "p2p")
 struct ShardBlob {  // what a rank publishes to the others (ICG_SHARD_BLOB_BYTES)
     uint64_t magic, pid, ptr, doubles;
@@ -3126,10 +2895,6 @@ int icg_ba_shard_export(icg_ba *h, int rank, int world, uint8_t *blob) {
     if (!h || !blob) {
         set_error("icg_ba_shard_export: bad arguments");
         return ICG_EINVAL;
-    }
-    if (h->comm) {
-        nccl_api().CommDestroy((ncclComm_t) h->comm);
-        h->comm = nullptr;
     }
     int rc = split_setup(h, rank, world);
     if (rc != ICG_OK) return rc;

@@ -19,9 +19,9 @@
 //   every rank   ba_accept_split  waits for the G slots, sums them in rank order: identical inputs -> identical accept / reject, radius and
 //                                 termination decisions on every rank, no broadcast of the LM state
 //
-// Three flag synchronisations per attempt, no NCCL on the data path, no host round trip.  The flags are monotonically increasing epoch
-// counters (one per LM attempt over the life of the handle); a consumer that does not see its flag within ~2 s raises the handle's
-// device-side error word instead of hanging the GPU.
+// Three flag synchronisations per attempt, no collective library on the data path, no host round trip.  The flags are monotonically
+// increasing epoch counters (one per LM attempt over the life of the handle); a consumer that does not see its flag within ~2 s raises the
+// handle's device-side error word instead of hanging the GPU.
 #pragma once
 #include <cooperative_groups.h>
 
@@ -545,7 +545,8 @@ __global__ void __launch_bounds__(SOLVE_THREADS) ba_solve_cam(BaCaps C, BaDev D,
 //   (3) cluster barrier (the stores have landed); the right-hand-side row's entries of the panel are y = L^-1 rhs.
 // Backward substitution L^T x = y, distributed: tile rows last to first; the owner of tile row T solves the 8 x 8 triangle (one warp), adds the
 // row's contributions to its own partial sums for the columns on the left and pushes the partial sums of the next three tile rows (final by
-// construction: its next own tile row is T - 4) to their owners' inboxes; one cluster barrier per tile row.
+// construction: its next own tile row is T - 4) to their owners' inboxes by st.async; the owner's inbox mbarrier counts the bytes, no cluster
+// barrier per tile row.
 constexpr int DSM_CL = 4;
 static_assert(SOLVE_THREADS == 256 && DSM_CL == SPLIT_CLUSTER, "ba_solve_cam_dsm: warp r assembles row r of a tile row; one launch geometry for both forms");
 __host__ __device__ inline int dsm_tile_off(int cr, int m) { return m * cr + 2 * m * (m - 1); }  // tiles ahead of local tile row m (T = cr + 4 m)
@@ -573,9 +574,6 @@ __device__ __forceinline__ void dsm_mbar_arrive_local(unsigned bar) { asm volati
 __device__ __forceinline__ void dsm_mbar_arrive_expect_tx_remote(unsigned bar_cluster, unsigned tx) {
     asm volatile("mbarrier.arrive.expect_tx.release.cluster.shared::cluster.b64 _, [%0], %1;" ::"r"(bar_cluster), "r"(tx) : "memory");
 }
-__device__ __forceinline__ void st_async_v2(unsigned dst_cluster, double a, double b, unsigned bar_cluster) {
-    asm volatile("st.async.weak.shared::cluster.mbarrier::complete_tx::bytes.v2.f64 [%0], {%1, %2}, [%3];" ::"r"(dst_cluster), "d"(a), "d"(b), "r"(bar_cluster) : "memory");
-}
 __device__ __forceinline__ void st_async_f64(unsigned dst_cluster, double a, unsigned bar_cluster) {
     asm volatile("st.async.weak.shared::cluster.mbarrier::complete_tx::bytes.f64 [%0], %1, [%2];" ::"r"(dst_cluster), "d"(a), "r"(bar_cluster) : "memory");
 }
@@ -598,11 +596,9 @@ __device__ __forceinline__ void dsm_mbar_wait(unsigned bar, unsigned parity, vol
     }
 }
 
-// variant: hand-over with asynchronous stores (st.async) + mbarriers carrying transaction counts instead of a cluster barrier -- bit 0: of the
-// panel column, bit 1: of the back-substitution's partial sums.  Measured (profiles/r2_ba_solve_cam_dsm.md): the panel hand-over is bound by the
-// SM-to-SM bandwidth either way and the cluster barrier is the cheaper form there; the back-substitution chain gains 15 % from the point-to-point form.
-constexpr int DSM_V_MBAR_PANEL = 1, DSM_V_MBAR_BSUB = 2;
-__global__ void __launch_bounds__(SOLVE_THREADS, 1) ba_solve_cam_dsm(BaCaps C, BaDev D, unsigned long long epoch, int variant) {
+// Hand-over forms, measured (profiles/r2_ba_solve_cam_dsm.md): the panel column is bound by the SM-to-SM bandwidth, and st.async + mbarriers
+// were no cheaper there than plain stores + the cluster barrier; in the back-substitution chain the point-to-point form gains 15 %.
+__global__ void __launch_bounds__(SOLVE_THREADS, 1) ba_solve_cam_dsm(BaCaps C, BaDev D, unsigned long long epoch) {
     extern __shared__ double sm[];
     cg::cluster_group cluster = cg::this_cluster();
     constexpr int CL = DSM_CL;
@@ -611,7 +607,6 @@ __global__ void __launch_bounds__(SOLVE_THREADS, 1) ba_solve_cam_dsm(BaCaps C, B
     if (w % D.world != D.rank) return;   // uniform over the cluster
     LmState &st = D.st[w];
     if (st.done) return;
-    const bool use_mbar = variant & DSM_V_MBAR_PANEL, bsub_mbar = variant & DSM_V_MBAR_BSUB;
     const WinDims dm = D.dims[w];
     const int K = dm.K, NCV = 6 * K + 7, N = 15 * K + 7, NR = N + 1;
     const int ntc = dsm_ntiles(C.N + 1), VL = ntc * 8;   // capacity: tiles per side, vector length
@@ -632,8 +627,8 @@ __global__ void __launch_bounds__(SOLVE_THREADS, 1) ba_solve_cam_dsm(BaCaps C, B
     double *s_dv = s_Lf + 64;                 // 8: its reciprocal pivots
     double *s_inbox = s_dv + 8;               // [CL][8]
     double *s_xT = s_inbox + 8 * CL;          // 8
-    int *s_fail = (int *) (s_xT + 8);         // [0] breakdown, [1] a bounded wait ran out; then the mbarriers (8 doubles reserved)
-    unsigned long long *s_bar = (unsigned long long *) (s_xT + 12);  // [0], [1]: panel column by parity; [2]: back-substitution inbox
+    int *s_fail = (int *) (s_xT + 8);         // [0] breakdown, [1] a bounded wait ran out; then the mbarrier (8 doubles reserved)
+    unsigned long long *s_bar = (unsigned long long *) (s_xT + 12);  // the back-substitution inbox's mbarrier
     double *s_dg = s_xT + 16;                 // [ntc][64] replicated diagonal tiles
     double *s_P = s_dg + (size_t) ntc * 64;   // [2][ntc][64] panel column, by panel parity
     double *s_tiles = s_P + (size_t) 2 * ntc * 64;
@@ -657,7 +652,7 @@ __global__ void __launch_bounds__(SOLVE_THREADS, 1) ba_solve_cam_dsm(BaCaps C, B
     if (tid < 8 * CL) s_inbox[tid] = 0;
     if (tid == 0) {
         s_fail[0] = 0, s_fail[1] = 0;
-        dsm_mbar_init(smem_u32(s_bar), CL), dsm_mbar_init(smem_u32(s_bar + 1), CL), dsm_mbar_init(smem_u32(s_bar + 2), CL - 1);
+        dsm_mbar_init(smem_u32(s_bar), CL - 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     __syncthreads();
@@ -770,10 +765,7 @@ __global__ void __launch_bounds__(SOLVE_THREADS, 1) ba_solve_cam_dsm(BaCaps C, B
         const double *PJ = s_P + (size_t) ((J - 1) & 1) * ntc * 64;   // panel J - 1's solved rows (J > 0)
         const unsigned long long tc0 = DSM_NOW();
         (void) tc0;
-        if (J > 0) {
-            if (use_mbar) dsm_mbar_wait(smem_u32(s_bar + ((J - 1) & 1)), ((J - 1) >> 1) & 1, s_dead, D.S.err);   // panel J - 1's column has landed
-            if (tid < 8 && Tn > J - 1) s_y[8 * (J - 1) + tid] = PJ[(size_t) Tn * 64 + rn * 8 + tid];         // its right-hand-side entries: y
-        }
+        if (J > 0 && tid < 8 && Tn > J - 1) s_y[8 * (J - 1) + tid] = PJ[(size_t) Tn * 64 + rn * 8 + tid];   // panel J - 1's right-hand-side entries: y
         DSM_CLK2(0, tc0)  // wait for the panel column
         const unsigned long long tc1 = DSM_NOW();
         (void) tc1;
@@ -931,33 +923,14 @@ __global__ void __launch_bounds__(SOLVE_THREADS, 1) ba_solve_cam_dsm(BaCaps C, B
                 double *dstP = s_P + (size_t) (J & 1) * ntc * 64 + (size_t) T * 64 + r * 8;
 #pragma unroll
                 for (int c = 0; c < 8; c += 2) *(double2 *) (tp + c) = make_double2(x[c], x[c + 1]);
-                if (use_mbar) {
-                    const unsigned a0 = smem_u32(dstP), b0 = smem_u32(s_bar + (J & 1));
 #pragma unroll
-                    for (int q = 0; q < CL; q++) {
-                        const unsigned ap = mapa_u32(a0, q), ab = mapa_u32(b0, q);
+                for (int q = 0; q < CL; q++) {
+                    double *rp = cluster.map_shared_rank(dstP, q);
 #pragma unroll
-                        for (int c = 0; c < 8; c += 2) st_async_v2(ap + 8u * c, x[c], x[c + 1], ab);
-                    }
-                } else {
-#pragma unroll
-                    for (int q = 0; q < CL; q++) {
-                        double *rp = cluster.map_shared_rank(dstP, q);
-#pragma unroll
-                        for (int c = 0; c < 8; c += 2) *(double2 *) (rp + c) = make_double2(x[c], x[c + 1]);
-                    }
+                    for (int c = 0; c < 8; c += 2) *(double2 *) (rp + c) = make_double2(x[c], x[c + 1]);
                 }
             }
-            if (use_mbar) {
-                // every CTA arrives on every CTA's barrier of this panel (also with nothing sent: the arrival says "I am done reading the
-                // buffer of panel J - 1", which the receiver's next-but-one panel overwrites) and announces its bytes
-                if (tid < CL) {
-                    const int nloc = cr + CL * m0 < nt ? (nt - 1 - (cr + CL * m0)) / CL + 1 : 0;   // local tile rows below the panel
-                    dsm_mbar_arrive_expect_tx_remote(mapa_u32(smem_u32(s_bar + (J & 1)), tid), 512u * nloc);
-                }
-            } else {
-                cluster.sync();
-            }
+            cluster.sync();
         }
         DSM_CLK(3, tc2)  // row solves + hand-over
     }
@@ -968,7 +941,6 @@ __global__ void __launch_bounds__(SOLVE_THREADS, 1) ba_solve_cam_dsm(BaCaps C, B
     if (valid) {
         {   // the last panel's column (only the right-hand-side row can be below it)
             const int J = npan - 1;
-            if (use_mbar) dsm_mbar_wait(smem_u32(s_bar + (J & 1)), (J >> 1) & 1, s_dead, D.S.err);
             if (tid < 8 && Tn > J) s_y[8 * J + tid] = s_P[(size_t) (J & 1) * ntc * 64 + (size_t) Tn * 64 + rn * 8 + tid];
         }
         if (rn > 0 && tid == 0) {   // the right-hand-side row shares the last diagonal tile with the last rn columns
@@ -1005,12 +977,10 @@ __global__ void __launch_bounds__(SOLVE_THREADS, 1) ba_solve_cam_dsm(BaCaps C, B
 #pragma unroll
                         for (int r = 0; r < 8; r++) tcr[r] = 0;
                     }
-                    if (bsub_mbar) {
-                        // three messages per tile row (from the owners of T + 1 .. T + 3); the ones that do not exist are arrived here
-                        const int nmiss = max(0, 3 - (npan - 1 - T));
-                        if (lane < nmiss) dsm_mbar_arrive_local(smem_u32(s_bar + 2));
-                        dsm_mbar_wait(smem_u32(s_bar + 2), ((npan - 1 - T) / CL) & 1, s_dead, D.S.err);
-                    }
+                    // three messages per tile row (from the owners of T + 1 .. T + 3); the ones that do not exist are arrived here
+                    const int nmiss = max(0, 3 - (npan - 1 - T));
+                    if (lane < nmiss) dsm_mbar_arrive_local(smem_u32(s_bar));
+                    dsm_mbar_wait(smem_u32(s_bar), ((npan - 1 - T) / CL) & 1, s_dead, D.S.err);
                     double v = 0;
                     if (lane < nbT) {
                         v = s_y[8 * T + c] - s_contrib[8 * T + c];
@@ -1030,13 +1000,9 @@ __global__ void __launch_bounds__(SOLVE_THREADS, 1) ba_solve_cam_dsm(BaCaps C, B
                     if (lane < ncrit) {
                         s_contrib[col] = acc;
                         const int q = (col >> 3) % CL;
-                        if (bsub_mbar) {
-                            const unsigned abar = mapa_u32(smem_u32(s_bar + 2), q);
-                            st_async_f64(mapa_u32(smem_u32(s_inbox + cr * 8 + (col & 7)), q), acc, abar);
-                            if ((col & 7) == 0) dsm_mbar_arrive_expect_tx_remote(abar, 64u);
-                        } else {
-                            cluster.map_shared_rank(s_inbox, q)[cr * 8 + (col & 7)] = acc;
-                        }
+                        const unsigned abar = mapa_u32(smem_u32(s_bar), q);
+                        st_async_f64(mapa_u32(smem_u32(s_inbox + cr * 8 + (col & 7)), q), acc, abar);
+                        if ((col & 7) == 0) dsm_mbar_arrive_expect_tx_remote(abar, 64u);
                     }
                 }
                 __syncthreads();
@@ -1049,7 +1015,6 @@ __global__ void __launch_bounds__(SOLVE_THREADS, 1) ba_solve_cam_dsm(BaCaps C, B
                 }
                 __syncthreads();
             }
-            if (!bsub_mbar) cluster.sync();
         }
     }
     cluster.sync();  // the solution has landed on CTA 0; no CTA leaves while its shared memory may still be written

@@ -30,7 +30,7 @@ extern "C" {
 #define ICG_ECUDA (-3)      /* CUDA runtime error (see icg_last_error) */
 #define ICG_EUNSUPPORTED (-4) /* parameter combination the sm_100a kernels are not built for */
 #define ICG_ENOMEM (-5)
-#define ICG_ENCCL (-6)
+/* (-6) is retired: do not reuse it */
 
 #define ICG_OPTFLOW_USE_INITIAL_FLOW 4 /* == cv::OPTFLOW_USE_INITIAL_FLOW */
 
@@ -384,30 +384,20 @@ typedef struct icg_ba_cull_output {
 } icg_ba_cull_output;
 int icg_ba_outlier_culling_resident(icg_ba *h, int n_windows, const icg_ba_problem *problems, const icg_ba_cull_input *in, icg_ba_cull_output *out);
 /*
- * Landmark sharding of the window solve across the GPUs of one box (SURVEY.md 8e): every process (one per GPU) uploads the same
- * camera-side problem but only ITS landmarks and their reprojection factors; per LM attempt one NCCL sum all-reduce of the packed
- * [vision Gram matrix + gradient | Schur term | vision cost, sum rho^2] buffer (+ an n-double max / 4n-double sum) makes the
- * reduced camera system identical on all ranks, which then factorise it redundantly (deterministic, no broadcast) and
- * back-substitute their own landmarks.  Camera-only factors (IMU, GNSS, priors) are evaluated by every rank and counted on rank 0.
- * icg_nccl_unique_id: rank 0 creates the 128-byte ncclUniqueId, the caller distributes it (e.g. torch.distributed broadcast);
- * icg_ba_set_shard(world = 1) returns the handle to single-GPU operation.  NCCL is dlopen-ed (libnccl.so.2) on first use.
- */
-int icg_nccl_unique_id(uint8_t *id128);
-int icg_ba_set_shard(icg_ba *h, int rank, int world, const uint8_t *id128);
-/*
- * The same sharding over PEER MEMORY instead of NCCL (transport "p2p"; the faster path, and the only one for windows whose reduced
- * system does not fit one CTA, max_K > 14): window w of the batch is owned by rank w mod world.  Every rank STORES its packed reduction
- * operand straight into the owner's inbox over NVLink; the owner sums the `world` slots in rank order while assembling the reduced camera
- * system (the reduction is fused into the consumer, no collective kernel), solves it on a thread-block cluster and stores the camera
- * step into every rank's step buffer; a 5-scalar all-to-all closes the attempt.  Three release/acquire flag synchronisations per LM
- * attempt, no host round trip, deterministic (fixed summation order, independent of arrival order).
+ * Landmark sharding of the window solve across the GPUs of one box (SURVEY.md 8e), over PEER MEMORY: every process (one per GPU) uploads
+ * the same camera-side problem but only ITS landmarks and their reprojection factors; window w of the batch is owned by rank w mod world.
+ * Every rank STORES its packed reduction operand straight into the owner's inbox over NVLink; the owner sums the `world` slots in rank
+ * order while assembling the reduced camera system (the reduction is fused into the consumer, no collective kernel), evaluates the
+ * camera-only factors, solves the system on a thread-block cluster and stores the camera step into every rank's step buffer; a 5-scalar
+ * all-to-all closes the attempt.  Three release/acquire flag synchronisations per LM attempt, no host round trip, deterministic (fixed
+ * summation order, independent of arrival order).
  *   icg_ba_shard_export : allocates this rank's exchange buffer for a group of `world` ranks (<= 8, one box) and writes the
  *                         ICG_SHARD_BLOB_BYTES blob the other ranks need (CUDA IPC handle + process-local pointer);
  *   icg_ba_shard_connect: blobs = world x ICG_SHARD_BLOB_BYTES in rank order (the caller gathers them, e.g. torch.distributed
  *                         all_gather_object); handles living in the same process are connected by pointer (peer access enabled);
  *   icg_ba_shard_error  : non-zero if a flag wait timed out (a rank did not enqueue the same sequence).
  * All ranks must create their handles with the same max_windows and max_K and call the solve entry points with the same arguments.
- * icg_ba_set_shard(h, 0, 1, NULL) returns the handle to single-GPU operation.
+ * Once a handle has called icg_ba_shard_export it stays on this pipeline until it is destroyed.
  */
 #define ICG_SHARD_BLOB_BYTES 128
 int icg_ba_shard_export(icg_ba *h, int rank, int world, uint8_t *blob);

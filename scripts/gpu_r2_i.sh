@@ -1,5 +1,5 @@
 #!/bin/bash
-# Round-2 single-GPU session I: split-pipeline tests, cfg-4 stage profile + phase clocks (default variant and variants 0 / 3), full GPU suite, short bench.
+# Round-2 single-GPU session I: split-pipeline tests, cfg-4 stage profile + phase clocks, full GPU suite, short bench.
 set -u
 T=${1:-r2i}
 O=gpurun_out
@@ -9,11 +9,6 @@ tail -5 $O/${T}_pytest_split.log
 ICG_BA_PROFILE=1 timeout 200 python scripts/prof_ba.py 32 3 20 2000 > $O/${T}_ba_stages_cfg4.log 2>&1
 ICG_LIB_VARIANT=prof ICG_BA_PROFILE=1 timeout 200 python scripts/prof_ba.py 32 3 20 2000 > $O/${T}_ba_phase_clocks_cfg4.log 2>&1
 tail -22 $O/${T}_ba_stages_cfg4.log; sed -n '/ba_solve_cam_dsm phases/,$p' $O/${T}_ba_phase_clocks_cfg4.log
-for v in 3; do
-  ICG_BA_DSM_VARIANT=$v ICG_BA_PROFILE=1 timeout 120 python scripts/prof_ba.py 32 3 20 2000 > $O/${T}_stages_v$v.log 2>&1
-  ICG_BA_DSM_VARIANT=$v ICG_LIB_VARIANT=prof ICG_BA_PROFILE=1 timeout 120 python scripts/prof_ba.py 32 3 20 2000 > $O/${T}_clocks_v$v.log 2>&1
-  echo "== variant $v"; grep -E "  solve" $O/${T}_stages_v$v.log | tail -1; sed -n '/ba_solve_cam_dsm phases/,$p' $O/${T}_clocks_v$v.log
-done
 timeout 900 python -m pytest tests -q -m gpu > $O/${T}_pytest.log 2>&1; echo "pytest rc=$?" | tee -a $O/${T}_pytest.log
 tail -4 $O/${T}_pytest.log
 timeout 200 python __graft_entry__.py --smoke > $O/${T}_smoke.log 2>&1; echo "smoke rc=$?" | tee -a $O/${T}_smoke.log

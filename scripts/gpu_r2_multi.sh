@@ -1,5 +1,5 @@
 #!/bin/bash
-# Multi-GPU session: sharded-solve parity tests (spawn, p2p + nccl transports) and the bench at N ranks.  usage: scripts/gpu_r2_multi.sh <tag> <N>
+# Multi-GPU session: sharded-solve parity tests (spawn, p2p transport) and the bench at N ranks.  usage: scripts/gpu_r2_multi.sh <tag> <N>
 set -u
 T=${1:-r2m}
 N=${2:-2}

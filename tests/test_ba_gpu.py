@@ -488,18 +488,3 @@ def test_small_factor_seams_match_oracle(olib, solver):
         l = {0: 6, 1: 9, 2: 6, 3: 1}[int(t)]
         assert np.array_equal(J[:, :l], J0[:, col:col + l]) and (J.shape[1] == l or np.all(J[:, l:] == 0))
         col += l
-
-
-def test_nccl_transport_is_refused_for_split_pipeline_sizes():
-    """windows whose reduced camera system does not fit one CTA (max_K = 20) are sharded over peer memory only: icg_ba_set_shard(world > 1)
-    must say so instead of building an NCCL communicator it cannot use"""
-    from ic_gvins_b200._lib import IcgError, check, lib
-    from ic_gvins_b200.ba import WindowSolver
-    s = WindowSolver(max_windows=1, max_K=20, max_L=64, max_F=256, max_gnss=4, max_marg_r=1)
-    try:
-        import ctypes as C
-        idbuf = (C.c_uint8 * 128)()
-        with pytest.raises(IcgError, match="split pipeline"):
-            check(lib().icg_ba_set_shard(s._h, 0, 2, idbuf), "icg_ba_set_shard")
-    finally:
-        s.close()

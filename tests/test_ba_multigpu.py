@@ -101,13 +101,13 @@ def _run(world, cfg, transport):
 @pytest.mark.parametrize("world", [2, 0])  # 0 = min(8, all GPUs of the box)
 def test_sharded_cfg4_matches_oracle(world):
     """cfg 4 (20 KF / 2000 landmarks): the reduced camera system does not fit one CTA, so the handle runs the split pipeline and the shards talk
-    over peer memory (CUDA IPC, transport p2p); the NCCL transport is refused for these sizes (tests/test_ba_gpu.py)."""
+    over peer memory (CUDA IPC, transport p2p)."""
     n = _ngpu()
     world = world or min(8, n)
     _run(world, (20, 2000, 3), "p2p")
 
 
 @pytest.mark.skipif(_ngpu() < 2, reason="needs >= 2 GPUs")
-@pytest.mark.parametrize("transport", ["p2p", "nccl"])
+@pytest.mark.parametrize("transport", ["p2p"])
 def test_sharded_cfg3_matches_oracle(transport):
     _run(2, (10, 300, 2), transport)
